@@ -8,16 +8,22 @@ pass of those four kernels over one batch.  `value` is BASELINE.json's metric it
 HBM bytes ((11D+6N)BLs, BASELINE.md section 3) over the time the scan forward and backward took inside the step (CUDA
 events around each kernel) - against the HBM roofline; the whole block including the conv kernels is the side key `block`.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--dtype fp32|bf16] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dtype fp32|bf16] [--impl ours|reference] [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes what the last timed step computed (rank 0) as DIR/<name>.npy in float32: the results a caller of
+the four ops receives (conv_out, scan_out, du, ddelta, dA, dB, dC, dD, dz, ddelta_bias, dx, dweight, dbias; not the saved-state
+checkpoint, whose layout is private to the kernels).  The (batch, channel)-by-L tensors are cut to a fixed, seeded sample of
+DUMP_ROWS rows so the dump stays near 30 MB; the inputs are seeded too, so two builds run with the same arguments can be
+compared output for output.
 
 N > 1 is launched by torchrun (one rank per GPU); every rank runs its own batch (weak scaling, no data-path collective:
 every (batch, channel) scan lane is independent - SURVEY.md section 8e); time = max over ranks, value = sum of bytes / time.
 
 `--impl reference` times the CPU path for the SAME step - same B, D, L, N, the same number of steps and warm-up steps - on
 all host cores: the C/OpenMP restatement of the reference's selective_scan_ref / causal_conv1d_ref algorithm
-(oracle/scan_oracle.c, kind "port"; /root/reference does not exist on the GPU box and its pure-PyTorch loop needs ~17 s per
-full-config step).  The pure-PyTorch form (oracle/torch_ref.py, the reference's own arithmetic op for op) is timed on a bounded
-sample and reported beside it as `pytorch_ref_sample`, labelled as a sample.
+(oracle/scan_oracle.c, kind "port"; the reference's pure-PyTorch loop needs ~17 s per full-config step).  The pure-PyTorch
+form (oracle/torch_ref.py, the reference's own arithmetic op for op) is timed on a bounded sample and reported beside
+it as `pytorch_ref_sample`, labelled as a sample.
 """
 from __future__ import annotations
 
@@ -64,6 +70,22 @@ def make_inputs(batch, dtype, device, seed=0, pin=False):
         t = {k: v.to(device) for k, v in t.items()}
     w = {k: v.to(device) for k, v in w.items()}
     return t, w
+
+
+DUMP_ROWS = 256
+GRAD_NAMES = ("du", "ddelta", "dA", "dB", "dC", "dD", "dz", "ddelta_bias")      # ops.selective_scan_bwd's results, in order
+
+
+def dump_outputs(outdir, outs):
+    """Writes outs (name -> tensor) as outdir/<name>.npy in float32.  A (B, D, L) tensor keeps only DUMP_ROWS of its B*D rows,
+    the same seeded sample (in ascending row order) for every tensor and every run."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    rows = torch.randperm(B * D, generator=torch.Generator().manual_seed(1234))[:DUMP_ROWS].sort().values
+    for name, v in outs.items():
+        if v.shape[:2] == (B, D) and v.dim() == 3:
+            v = v.reshape(B * D, -1)[rows.to(v.device)]
+        np.save(os.path.join(outdir, name + ".npy"), v.detach().float().cpu().numpy())
 
 
 class ClockSampler(threading.Thread):
@@ -319,7 +341,12 @@ def main():
     ap.add_argument("--train-batch", type=int, default=16, help="GLOBAL batch of the 512x512 training leg (BASELINE configs[2]); split over the ranks")
     ap.add_argument("--train-size", type=int, default=512)
     ap.add_argument("--no-hires", action="store_true", help="skip the 1024x1024 / global batch 8 training leg (BASELINE configs[3])")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path: use it with --impl ours")
     quiet_stdout()
     if args.impl == "reference":
         return run_reference(args)
@@ -354,9 +381,9 @@ def main():
         g = ops.selective_scan_bwd(u, t["delta"], w["A"], t["Bm"], t["Cm"], w["Dp"], t["z"], w["dbias"], t["dout"], xs, True,
                                    du=du, ddelta=dd, dz=dz)
         if e: e[3].record()
-        ops.causal_conv1d_bwd(t["x"], w["cw"], w["cb"], du, True, dx=dx)
+        _, dw, db = ops.causal_conv1d_bwd(t["x"], w["cw"], w["cb"], du, True, dx=dx)
         if e: e[4].record()
-        return g
+        return {"conv_out": u, "scan_out": out, **dict(zip(GRAD_NAMES, g)), "dx": dx, "dweight": dw, "dbias": db}
 
     for _ in range(warm):
         step()
@@ -371,7 +398,11 @@ def main():
     start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     start.record()
     for i in range(args.steps):
-        step(ev[i])
+        outs = step(ev[i])
+        if i + 1 < args.steps:
+            # freed before the next step allocates, so every timed step gets the same buffer placement; outputs kept
+            # alive across steps move the scan's buffers to other addresses, which slows the scan forward
+            del outs
     stop.record()
     torch.cuda.synchronize()
     if dist: dist.barrier()
@@ -381,6 +412,9 @@ def main():
     dev_ms = start.elapsed_time(stop)
     dev_ms = reduce_max_ms(dev_ms, dist, dev)
     per_kernel = {n: sum(ev[i][k].elapsed_time(ev[i][k + 1]) for i in range(args.steps)) / args.steps for k, n in enumerate(names)}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs)
+    del outs
 
     # ---------------- end-to-end arm: public autograd API, pinned host buffers, H2D + D2H inside the timed region ---
     # Every step copies ITS inputs from pinned host memory and reads its loss back.  The copies run on a second stream into
