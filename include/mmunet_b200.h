@@ -272,6 +272,55 @@ int mmu_mamba_narrow_post_bwd(const mmu_narrow_params *p, void *stream);
 int mmu_mamba_narrow_pre_bwd(const mmu_narrow_params *p, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Deterministic mode.  Every entry point above that sums floats across CTAs does it with fp32 atomics, so those sums differ in
+ * the last bits from run to run.  The _det variants below compute the same results without floating-point atomics: each CTA
+ * stores its partial sums to a slot of the caller's workspace indexed by its work item (row group, batch, segment, token block,
+ * pixel block), and one ordered-reduce kernel adds the slots, in a fixed order, into the same outputs.  For the same inputs,
+ * shapes, strides, dtypes, library build, MMU_* knobs and device, every output is then bitwise identical from call to call,
+ * on any stream and in CUDA-graph replays.
+ *   - Arguments are those of the plain entry point plus `ws` / `ws_bytes`: a caller-allocated device workspace (256-byte
+ *     aligned; its contents on entry do not matter) of at least the size the matching ..._det_workspace() query returns.  The
+ *     query is a pure host function: an upper bound for whichever kernel the dispatcher picks for that shape.
+ *   - MMU_ERR_WORKSPACE when ws is NULL or smaller than that, before any work is enqueued.
+ *   - The accumulate-into contract is unchanged: the caller zero-fills the accumulated outputs, the kernels add into them.
+ *   - mmu_deterministic_default(): 1 when the environment knob MMU_DETERMINISTIC is a non-zero integer (read once, like the other
+ *     MMU_* knobs), for callers that select the mode without an API of their own.
+ * --------------------------------------------------------------------------------------------- */
+int32_t mmu_deterministic_default(void);
+
+/* selective scan backward.  Partials: dB and dC as [row group][batch][dstate][seqlen] (the sums over the rows of one CTA), dA as
+ * [batch][segment][dim][dstate], dD and ddelta_bias as [batch][segment][dim].  The opt-in v4 kernels are never used here.
+ * The workspace grows with batch * ceil(dim / rows per CTA) * dstate * seqlen * 8 bytes; callers slice the batch to bound it. */
+size_t mmu_selective_scan_bwd_det_workspace(int32_t batch, int32_t dim, int32_t seqlen, int32_t dstate);
+int mmu_selective_scan_bwd_det(const mmu_scan_bwd_params *p, void *ws, size_t ws_bytes, void *stream);
+/* causal conv1d backward.  Partials [batch][token block][dim][5] (4 width-padded taps | bias). */
+size_t mmu_causal_conv1d_bwd_det_workspace(int32_t batch, int32_t dim, int32_t seqlen, int32_t dtype);
+int mmu_causal_conv1d_bwd_det(const mmu_conv_params *p, void *ws, size_t ws_bytes, void *stream);
+/* narrow Mamba block backward.  Partials [batch][256-token tile][floats]: post_bwd the out_proj | d(altho) block of dweights,
+ * pre_bwd every float of dweights before out_proj. */
+size_t mmu_mamba_narrow_post_bwd_det_workspace(int32_t batch, int32_t seqlen);
+size_t mmu_mamba_narrow_pre_bwd_det_workspace(int32_t batch, int32_t seqlen);
+int mmu_mamba_narrow_post_bwd_det(const mmu_narrow_params *p, void *ws, size_t ws_bytes, void *stream);
+int mmu_mamba_narrow_pre_bwd_det(const mmu_narrow_params *p, void *ws, size_t ws_bytes, void *stream);
+/* channels-last GroupNorm.  Partials [B][pixel block][G][2] (forward statistics, reduced into `sums`) and [B][pixel block][G][10]
+ * (backward: S1, S2, dgamma[4], dbeta[4]). */
+size_t mmu_group_norm_nhwc_fwd_det_workspace(int32_t B, int32_t C, int32_t HW, int32_t G);
+size_t mmu_group_norm_nhwc_bwd_det_workspace(int32_t B, int32_t C, int32_t HW, int32_t G);
+int mmu_group_norm_nhwc_fwd_det(const void *x, const float *gamma, const float *beta, void *y, float *sums, float *mean, float *rstd,
+                                int32_t in_dtype, int32_t out_dtype, int32_t B, int32_t C, int32_t HW, int32_t G, float eps, void *ws,
+                                size_t ws_bytes, void *stream);
+int mmu_group_norm_nhwc_bwd_det(const void *x, const float *gamma, const void *dy, const float *mean, const float *rstd, void *dx,
+                                float *sums2, float *dgamma_dbeta, int32_t in_dtype, int32_t out_dtype, int32_t B, int32_t C, int32_t HW,
+                                int32_t G, void *ws, size_t ws_bytes, void *stream);
+/* snake sampler backward.  Gather-side: one thread owns a column of dfeat (b, channel(s), all rows, x) and walks the samples that read
+ * column x in a fixed order; dy is summed over all channels by one thread per sample.  Needs no workspace (the query returns 0,
+ * ws may be NULL). */
+size_t mmu_snake_sample_bwd_det_workspace(int32_t B, int32_t C, int32_t H, int32_t W, int32_t K, int32_t channels_last);
+int mmu_snake_sample_bwd_det(const void *feat, const float *y, const void *dout, float *dfeat, float *dy, int32_t in_dtype,
+                             int32_t out_dtype, int32_t B, int32_t C, int32_t H, int32_t W, int32_t K, int32_t channels_last, void *ws,
+                             size_t ws_bytes, void *stream);
+
+/* ---------------------------------------------------------------------------------------------
  * misc
  * --------------------------------------------------------------------------------------------- */
 int mmu_version(void);

@@ -28,7 +28,8 @@ int set_error(int code, const char *fmt, ...) {
 namespace {
 constexpr const char *kKnobNames[] = {
     "MMU_SCAN_V", "MMU_BWD_V", "MMU_FWD_CFG", "MMU_BWD_CFG", "MMU_FWD_NSEG", "MMU_BWD_NSEG", "MMU_NO_PREFETCH", "MMU_FWD3_LPR",
-    "MMU_FWD3_W", "MMU_BWD3_W", "MMU_BWD_CHAIN", "MMU_V4_WPSM", "MMU_V4_BWD_WPSM", "MMU_V4_MIN_DIM", "MMU_V5_MIN_DIM", "MMU_FUSE", "MMU_RING", "MMU_V5_W", "MMU_V5_MIN_WARPS", "MMU_RING_BF16"};
+    "MMU_FWD3_W", "MMU_BWD3_W", "MMU_BWD_CHAIN", "MMU_V4_WPSM", "MMU_V4_BWD_WPSM", "MMU_V4_MIN_DIM", "MMU_V5_MIN_DIM", "MMU_FUSE", "MMU_RING", "MMU_V5_W", "MMU_V5_MIN_WARPS", "MMU_RING_BF16",
+    "MMU_DETERMINISTIC"};
 constexpr int kNumKnobs = sizeof(kKnobNames) / sizeof(kKnobNames[0]);
 struct KnobTable {
     bool set[kNumKnobs];
@@ -69,4 +70,5 @@ extern "C" void mmu_reload_knobs(void) {
     mmu::load_knobs();
 }
 extern "C" const char *mmu_last_error(void) { return mmu::g_err; }
+extern "C" int32_t mmu_deterministic_default(void) { return mmu::knob("MMU_DETERMINISTIC", 0) != 0 ? 1 : 0; }
 extern "C" uint64_t mmu_launch_count(void) { return mmu::g_launches.load(std::memory_order_relaxed); }

@@ -24,6 +24,7 @@ struct ConvArgs {
     int silu, reverse;
     unsigned vec_mask;   // bit0 x, bit1 out/dx, bit2 dout
     OrdMap ord;          // fused scan order: x / dx live at ord(l), out / dout at l
+    float *part;         // deterministic backward: [b][token block][d][5] partials (4 taps, width-padded | bias)
 };
 
 constexpr int kConvNT = 128;
@@ -147,7 +148,8 @@ template <typename IN_T, bool ORD> __global__ void __launch_bounds__(kConvNT) co
                  rev, o);
 }
 
-template <typename IN_T, bool ORD> __global__ void __launch_bounds__(kConvNT) conv1d_bwd_kernel(const __grid_constant__ ConvArgs p) {
+// DET: the block's dw / db sums go to its own slot of p.part instead of atomics (the ordered reduce in det_reduce.cu adds them)
+template <typename IN_T, bool ORD, bool DET = false> __global__ void __launch_bounds__(kConvNT) conv1d_bwd_kernel(const __grid_constant__ ConvArgs p) {
     constexpr int kConvVT = ConvVT<IN_T>::value;
     const int d = blockIdx.y, b = blockIdx.z;
     const int t = (blockIdx.x * kConvNT + threadIdx.x) * kConvVT;
@@ -260,7 +262,9 @@ template <typename IN_T, bool ORD> __global__ void __launch_bounds__(kConvNT) co
         float v = 0.f;
 #pragma unroll
         for (int wdx = 0; wdx < kConvNT / 32; ++wdx) v += red[wdx][threadIdx.x];
-        if (threadIdx.x == 4) {
+        if constexpr (DET) {
+            p.part[(((int64_t)b * gridDim.x + blockIdx.x) * p.D + d) * 5 + threadIdx.x] = v;
+        } else if (threadIdx.x == 4) {
             if (p.db != nullptr) atomicAdd(p.db + d, v);
         } else {
             const int kk = (int)threadIdx.x - (4 - p.W);
@@ -270,8 +274,17 @@ template <typename IN_T, bool ORD> __global__ void __launch_bounds__(kConvNT) co
 }
 
 namespace {
-template <typename IN_T> int run_conv(const mmu_conv_params *p, bool bwd, cudaStream_t st) {
+template <typename IN_T> constexpr int conv_block_tokens() { return kConvNT * ConvVT<IN_T>::value; }
+
+// deterministic backward: the partial slots, [b][token block][d][5]
+size_t conv_det_floats(int B, int D, int L, int dtype) {
+    const int per_block = dtype == MMU_F32 ? conv_block_tokens<float>() : conv_block_tokens<__nv_bfloat16>();
+    return (size_t)B * ((L + per_block - 1) / per_block) * D * 5;
+}
+
+template <typename IN_T> int run_conv(const mmu_conv_params *p, bool bwd, float *part, cudaStream_t st) {
     ConvArgs a{};
+    a.part = part;
     a.x = p->x, a.dout = p->dout, a.w = p->weight, a.bias = p->bias, a.out = p->out, a.dx = p->dx;
     a.dw = p->dweight, a.db = p->dbias;
     a.x_bs = p->x_bs, a.x_ds = p->x_ds, a.o_bs = p->out_bs, a.o_ds = p->out_ds, a.w_ds = p->w_ds, a.w_ws = p->w_ws;
@@ -294,6 +307,19 @@ template <typename IN_T> int run_conv(const mmu_conv_params *p, bool bwd, cudaSt
     dim3 grid((L + per_block - 1) / per_block, p->dim, p->batch);
     if (grid.y > 65535 || grid.z > 65535) return set_error(MMU_ERR_UNSUPPORTED, "causal_conv1d: dim/batch > 65535");
     const bool ord = p->order != MMU_ORDER_ROWMAJOR;
+    if (bwd && part != nullptr) {
+        if (ord) conv1d_bwd_kernel<IN_T, true, true><<<grid, kConvNT, 0, st>>>(a);
+        else conv1d_bwd_kernel<IN_T, false, true><<<grid, kConvNT, 0, st>>>(a);
+        count_launch();
+        if (int rc = check_launch("causal_conv1d_bwd(deterministic)")) return rc;
+        const int64_t items = (int64_t)p->batch * grid.x;
+        // dweight[d][k] = sum of slot (d, 4 - W + k);  dbias[d] = sum of slot (d, 4)
+        if (int rc = det_reduce(DetSum{part + (4 - p->width), items, (int64_t)p->dim * 5, 1, p->dim, p->width, 0, 5, p->dweight, 0,
+                                       p->width, 1}, st))
+            return rc;
+        if (p->dbias == nullptr) return MMU_OK;
+        return det_reduce(DetSum{part + 4, items, (int64_t)p->dim * 5, 1, p->dim, 1, 0, 5, p->dbias, 0, 1, 0}, st);
+    }
     if (bwd) {
         if (ord) conv1d_bwd_kernel<IN_T, true><<<grid, kConvNT, 0, st>>>(a);
         else conv1d_bwd_kernel<IN_T, false><<<grid, kConvNT, 0, st>>>(a);
@@ -305,7 +331,7 @@ template <typename IN_T> int run_conv(const mmu_conv_params *p, bool bwd, cudaSt
     return check_launch(bwd ? "causal_conv1d_bwd" : "causal_conv1d_fwd");
 }
 
-int conv_entry(const mmu_conv_params *p, bool bwd, void *stream) {
+int conv_entry(const mmu_conv_params *p, bool bwd, float *part, void *stream) {
     if (p == nullptr) return set_error(MMU_ERR_INVALID, "causal_conv1d: null params");
     if (p->batch <= 0 || p->dim <= 0 || p->seqlen <= 0) return set_error(MMU_ERR_INVALID, "causal_conv1d: empty shape");
     if (p->width < 2 || p->width > 4) return set_error(MMU_ERR_INVALID, "causal_conv1d only supports width between 2 and 4");
@@ -315,14 +341,29 @@ int conv_entry(const mmu_conv_params *p, bool bwd, void *stream) {
     if (bwd && p->bias != nullptr && !p->dbias) return set_error(MMU_ERR_INVALID, "causal_conv1d_bwd: dbias missing");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     switch (p->dtype) {
-        case MMU_F32: return run_conv<float>(p, bwd, st);
-        case MMU_BF16: return run_conv<__nv_bfloat16>(p, bwd, st);
-        case MMU_F16: return run_conv<__half>(p, bwd, st);
+        case MMU_F32: return run_conv<float>(p, bwd, part, st);
+        case MMU_BF16: return run_conv<__nv_bfloat16>(p, bwd, part, st);
+        case MMU_F16: return run_conv<__half>(p, bwd, part, st);
         default: return set_error(MMU_ERR_UNSUPPORTED, "causal_conv1d: dtype %d", p->dtype);
     }
 }
 }  // namespace
 }  // namespace mmu
 
-extern "C" int mmu_causal_conv1d_fwd(const mmu_conv_params *p, void *stream) { return mmu::conv_entry(p, false, stream); }
-extern "C" int mmu_causal_conv1d_bwd(const mmu_conv_params *p, void *stream) { return mmu::conv_entry(p, true, stream); }
+extern "C" int mmu_causal_conv1d_fwd(const mmu_conv_params *p, void *stream) { return mmu::conv_entry(p, false, nullptr, stream); }
+extern "C" int mmu_causal_conv1d_bwd(const mmu_conv_params *p, void *stream) { return mmu::conv_entry(p, true, nullptr, stream); }
+
+extern "C" size_t mmu_causal_conv1d_bwd_det_workspace(int32_t batch, int32_t dim, int32_t seqlen, int32_t dtype) {
+    if (batch <= 0 || dim <= 0 || seqlen <= 0) return 0;
+    mmu::DetWs w{nullptr};
+    w.take(mmu::conv_det_floats(batch, dim, seqlen, dtype));
+    return w.used;
+}
+extern "C" int mmu_causal_conv1d_bwd_det(const mmu_conv_params *p, void *ws, size_t ws_bytes, void *stream) {
+    using namespace mmu;
+    if (p == nullptr) return set_error(MMU_ERR_INVALID, "causal_conv1d_bwd_det: null params");
+    const size_t need = mmu_causal_conv1d_bwd_det_workspace(p->batch, p->dim, p->seqlen, p->dtype);
+    if (need == 0) return set_error(MMU_ERR_INVALID, "causal_conv1d_bwd_det: empty shape");
+    if (int rc = det_ws_check(ws, ws_bytes, need, "causal_conv1d_bwd_det")) return rc;
+    return conv_entry(p, true, static_cast<float *>(ws), stream);
+}

@@ -17,6 +17,36 @@ void count_launch(int n = 1);
 int check_launch(const char *what);
 int knob(const char *name, int dflt);   // MMU_* tuning knob (environment, read once: capi.cu)
 
+// ---- deterministic mode (det_reduce.cu) -----------------------------------------------------------------------------------
+// Ordered sum over `items` partial slots, added into a strided destination: column (a, r, c), extents (n0, n1, n2);
+// src[i * item_stride + a * ss0 + r * ss1 + c], dst[a * ds0 + r * ds1 + c * ds2] += sum over i in a fixed order.
+struct DetSum {
+    const float *src;
+    int64_t items, item_stride;
+    int n0, n1, n2;
+    int64_t ss0, ss1;
+    float *dst;
+    int64_t ds0, ds1, ds2;
+};
+int det_reduce(const DetSum &r, cudaStream_t st);
+// Bump allocator over a caller's workspace: 256-byte aligned float slices.  size() of a dry run (base == nullptr) is the query.
+struct DetWs {
+    char *base;
+    size_t used = 0;
+    float *take(size_t floats) {
+        float *p = base ? reinterpret_cast<float *>(base + used) : nullptr;
+        used += (floats * sizeof(float) + 255) & ~(size_t)255;
+        return p;
+    }
+};
+// argument checks shared by every _det entry point: MMU_ERR_WORKSPACE when the caller's workspace is missing or too small
+inline int det_ws_check(const void *ws, size_t ws_bytes, size_t need, const char *what) {
+    if (need > 0 && (ws == nullptr || ws_bytes < need))
+        return set_error(MMU_ERR_WORKSPACE, "%s: deterministic workspace %zu < %zu bytes", what, ws ? ws_bytes : (size_t)0, need);
+    if (ws != nullptr && reinterpret_cast<uintptr_t>(ws) % 256 != 0) return set_error(MMU_ERR_INVALID, "%s: workspace must be 256-byte aligned", what);
+    return MMU_OK;
+}
+
 // ---- element conversion -----------------------------------------------------------------------
 template <typename T> struct Elem;
 template <> struct Elem<float> {

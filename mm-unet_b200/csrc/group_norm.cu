@@ -9,7 +9,8 @@
 //   backward: (1) per (b, group) S1 = sum gamma*dy, S2 = sum gamma*dy*xhat, per channel dgamma = sum dy*xhat, dbeta = sum dy
 //             (2) dx = rstd * (gamma*dy - (S1 + xhat*S2) / n)
 // All four kernels are single-pass HBM-bound streams; the partial sums are reduced in the block, then by fp32 atomics into
-// caller-zeroed accumulators.
+// caller-zeroed accumulators.  Deterministic mode (the _det entry points): the reduction kernels store the block sums to
+// [b][pixel block][G][2 | 10] slots instead, and the ordered reduce (det_reduce.cu) adds them into the same accumulators.
 #include "common.cuh"
 
 namespace mmu {
@@ -52,7 +53,7 @@ template <typename TI> __device__ __forceinline__ float gn_shift(const TI *group
 }
 
 // thread layout of the reduction kernels: tid = lane_p * G + g  (G | 256 or G >= 256 handled by the g loop)
-template <typename TI>
+template <typename TI, bool DET = false>
 __global__ void __launch_bounds__(kGnThreads) gn_stats_kernel(const TI *__restrict__ x, float *__restrict__ sums, GnGeom g) {
     extern __shared__ float sm[];                       // [2][kGnThreads]
     const int b = blockIdx.y, p0 = blockIdx.x * g.ppb, p1 = min(g.HW, p0 + g.ppb);
@@ -77,8 +78,13 @@ __global__ void __launch_bounds__(kGnThreads) gn_stats_kernel(const TI *__restri
         __syncthreads();
         if (lp == 0 && gi < G) {
             for (int l = 1; l < lanes; ++l) s += sm[l * G + (tid % G)], ss += sm[kGnThreads + l * G + (tid % G)];
-            atomicAdd(sums + ((int64_t)b * G + gi) * 2, s);
-            atomicAdd(sums + ((int64_t)b * G + gi) * 2 + 1, ss);
+            if constexpr (DET) {      // sums = the slots [b][pixel block][G][2]
+                float *slot = sums + (((int64_t)b * gridDim.x + blockIdx.x) * G + gi) * 2;
+                slot[0] = s, slot[1] = ss;
+            } else {
+                atomicAdd(sums + ((int64_t)b * G + gi) * 2, s);
+                atomicAdd(sums + ((int64_t)b * G + gi) * 2 + 1, ss);
+            }
         }
         __syncthreads();
     }
@@ -111,8 +117,8 @@ __global__ void __launch_bounds__(256) gn_apply_kernel(const TI *__restrict__ x,
     V4<TO>::st(y + bp * g.C + 4 * gi, o);
 }
 
-// backward reduction: sums2[b][g] = (S1, S2); dgb[c] = dgamma, dgb[C + c] = dbeta
-template <typename TI, typename TO>
+// backward reduction: sums2[b][g] = (S1, S2); dgb[c] = dgamma, dgb[C + c] = dbeta.  DET: sums2 = the slots [b][pixel block][G][10]
+template <typename TI, typename TO, bool DET = false>
 __global__ void __launch_bounds__(kGnThreads) gn_bwd_reduce_kernel(const TI *__restrict__ x, const TO *__restrict__ dy, const float *__restrict__ mean,
                                                                    const float *__restrict__ rstd, const float *__restrict__ gamma,
                                                                    float *__restrict__ sums2, float *__restrict__ dgb, GnGeom g) {
@@ -147,12 +153,18 @@ __global__ void __launch_bounds__(kGnThreads) gn_bwd_reduce_kernel(const TI *__r
             for (int l = 1; l < lanes; ++l)
 #pragma unroll
                 for (int k = 0; k < 10; ++k) acc[k] += sm[k * kGnThreads + l * G + (tid % G)];
-            atomicAdd(sums2 + ((int64_t)b * G + gi) * 2, acc[0]);
-            atomicAdd(sums2 + ((int64_t)b * G + gi) * 2 + 1, acc[1]);
+            if constexpr (DET) {
+                float *slot = sums2 + (((int64_t)b * gridDim.x + blockIdx.x) * G + gi) * 10;
 #pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                atomicAdd(dgb + 4 * gi + k, acc[2 + k]);
-                atomicAdd(dgb + g.C + 4 * gi + k, acc[6 + k]);
+                for (int k = 0; k < 10; ++k) slot[k] = acc[k];
+            } else {
+                atomicAdd(sums2 + ((int64_t)b * G + gi) * 2, acc[0]);
+                atomicAdd(sums2 + ((int64_t)b * G + gi) * 2 + 1, acc[1]);
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    atomicAdd(dgb + 4 * gi + k, acc[2 + k]);
+                    atomicAdd(dgb + g.C + 4 * gi + k, acc[6 + k]);
+                }
             }
         }
         __syncthreads();
@@ -184,15 +196,18 @@ __global__ void __launch_bounds__(256) gn_bwd_apply_kernel(const TI *__restrict_
 }
 
 namespace {
+// pixel blocks of the reduction grid: enough blocks to fill the GPU (~8 per SM), at least one pixel per lane
+int gn_pblocks(int B, int HW, int G) {
+    const int lanes = G >= kGnThreads ? 1 : kGnThreads / G;
+    return (int)std::min<int64_t>((HW + lanes - 1) / lanes, std::max<int64_t>(1, (148 * 8 + B - 1) / B));
+}
 int gn_geom(GnGeom &g, int B, int C, int HW, int G, float eps, dim3 &rgrid, dim3 &agrid) {
     if (B <= 0 || C <= 0 || HW <= 0 || G <= 0) return set_error(MMU_ERR_INVALID, "group_norm: bad shape B%d C%d HW%d G%d", B, C, HW, G);
     if (C != 4 * G) return set_error(MMU_ERR_UNSUPPORTED, "group_norm (channels-last): only 4 channels per group (C=%d, G=%d)", C, G);
     if (G < kGnThreads && kGnThreads % G != 0) return set_error(MMU_ERR_UNSUPPORTED, "group_norm: G=%d must divide %d or be >= it", G, kGnThreads);
     const int64_t items = (int64_t)HW * G;                      // per batch element
     if (items > 0x7fffffffLL || B > 65535) return set_error(MMU_ERR_UNSUPPORTED, "group_norm: problem too large");
-    // reduction grid: enough blocks to fill the GPU (~8 per SM), at least one pixel per lane
-    const int lanes = G >= kGnThreads ? 1 : kGnThreads / G;
-    int pblocks = (int)std::min<int64_t>((HW + lanes - 1) / lanes, std::max<int64_t>(1, (148 * 8 + B - 1) / B));
+    const int pblocks = gn_pblocks(B, HW, G);
     g = {B, C, HW, G, (HW + pblocks - 1) / pblocks, eps};
     rgrid = dim3((unsigned)((HW + g.ppb - 1) / g.ppb), (unsigned)B);
     agrid = dim3((unsigned)((items + 255) / 256), (unsigned)B);
@@ -208,20 +223,76 @@ int gn_geom(GnGeom &g, int B, int C, int HW, int G, float eps, dim3 &rgrid, dim3
     else if (in_dtype == MMU_BF16 && out_dtype == MMU_F32) { using TI = __nv_bfloat16; using TO = float; KERNEL_CALL; } \
     else return set_error(MMU_ERR_UNSUPPORTED, "group_norm: dtypes %d -> %d", in_dtype, out_dtype);
 
-extern "C" int mmu_group_norm_nhwc_fwd(const void *x, const float *gamma, const float *beta, void *y, float *sums, float *mean, float *rstd,
-                                       int32_t in_dtype, int32_t out_dtype, int32_t B, int32_t C, int32_t HW, int32_t G, float eps, void *stream) {
-    using namespace mmu;
+namespace mmu {
+namespace {
+// slots of the deterministic reductions: [b][pixel block][G][per]
+size_t gn_det_bytes(int B, int C, int HW, int G, int per) {
+    if (B <= 0 || C <= 0 || HW <= 0 || G <= 0) return 0;
+    DetWs w{nullptr};
+    w.take((size_t)B * gn_pblocks(B, HW, G) * G * per);
+    return w.used;
+}
+
+// part == nullptr: the atomic path; otherwise the block sums go to the slots `part` and are reduced into `sums` in order
+int gn_fwd(const void *x, const float *gamma, const float *beta, void *y, float *sums, float *mean, float *rstd, int32_t in_dtype,
+           int32_t out_dtype, int32_t B, int32_t C, int32_t HW, int32_t G, float eps, float *part, cudaStream_t st) {
     GnGeom g;
     dim3 rgrid, agrid;
     if (int rc = gn_geom(g, B, C, HW, G, eps, rgrid, agrid)) return rc;
     if (!x || !gamma || !beta || !y || !sums || !mean || !rstd) return set_error(MMU_ERR_INVALID, "group_norm_fwd: null pointer");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (in_dtype == MMU_F32) gn_stats_kernel<float><<<rgrid, kGnThreads, 2 * kGnThreads * sizeof(float), st>>>((const float *)x, sums, g);
-    else if (in_dtype == MMU_BF16) gn_stats_kernel<__nv_bfloat16><<<rgrid, kGnThreads, 2 * kGnThreads * sizeof(float), st>>>((const __nv_bfloat16 *)x, sums, g);
-    else return set_error(MMU_ERR_UNSUPPORTED, "group_norm: input dtype %d", in_dtype);
+    const size_t smem = 2 * kGnThreads * sizeof(float);
+    if (in_dtype == MMU_F32) {
+        if (part) gn_stats_kernel<float, true><<<rgrid, kGnThreads, smem, st>>>((const float *)x, part, g);
+        else gn_stats_kernel<float><<<rgrid, kGnThreads, smem, st>>>((const float *)x, sums, g);
+    } else if (in_dtype == MMU_BF16) {
+        if (part) gn_stats_kernel<__nv_bfloat16, true><<<rgrid, kGnThreads, smem, st>>>((const __nv_bfloat16 *)x, part, g);
+        else gn_stats_kernel<__nv_bfloat16><<<rgrid, kGnThreads, smem, st>>>((const __nv_bfloat16 *)x, sums, g);
+    } else {
+        return set_error(MMU_ERR_UNSUPPORTED, "group_norm: input dtype %d", in_dtype);
+    }
+    if (part) {
+        count_launch();
+        if (int rc = check_launch("group_norm_nhwc_fwd(deterministic)")) return rc;
+        if (int rc = det_reduce(DetSum{part, (int64_t)rgrid.x, (int64_t)G * 2, B, 1, 2 * G, (int64_t)rgrid.x * G * 2, 0, sums, 2 * G, 0, 1}, st))
+            return rc;
+    }
     MMU_GN_DISPATCH((gn_apply_kernel<TI, TO><<<agrid, 256, 0, st>>>((const TI *)x, sums, gamma, beta, (TO *)y, mean, rstd, g)))
-    count_launch(2);
+    count_launch(part ? 1 : 2);
     return check_launch("group_norm_nhwc_fwd");
+}
+
+int gn_bwd(const void *x, const float *gamma, const void *dy, const float *mean, const float *rstd, void *dx, float *sums2,
+           float *dgamma_dbeta, int32_t in_dtype, int32_t out_dtype, int32_t B, int32_t C, int32_t HW, int32_t G, float *part, cudaStream_t st) {
+    GnGeom g;
+    dim3 rgrid, agrid;
+    if (int rc = gn_geom(g, B, C, HW, G, 0.f, rgrid, agrid)) return rc;
+    if (!x || !gamma || !dy || !mean || !rstd || !dx || !sums2 || !dgamma_dbeta) return set_error(MMU_ERR_INVALID, "group_norm_bwd: null pointer");
+    const size_t smem = 10 * kGnThreads * sizeof(float);
+    if (part) {
+        MMU_GN_DISPATCH((gn_bwd_reduce_kernel<TI, TO, true><<<rgrid, kGnThreads, smem, st>>>(
+            (const TI *)x, (const TO *)dy, mean, rstd, gamma, part, dgamma_dbeta, g)))
+        count_launch();
+        if (int rc = check_launch("group_norm_nhwc_bwd(deterministic)")) return rc;
+        const int64_t nb = rgrid.x;
+        // sums2[b][g][0..1] = sum over pixel blocks of slot k = 0..1
+        if (int rc = det_reduce(DetSum{part, nb, (int64_t)G * 10, B, G, 2, nb * G * 10, 10, sums2, 2 * G, 2, 1}, st)) return rc;
+        // dgamma[4g + k] (slot 2 + k), dbeta[4g + k] (slot 6 + k): summed over batch and pixel blocks
+        if (int rc = det_reduce(DetSum{part + 2, (int64_t)B * nb, (int64_t)G * 10, 2, G, 4, 4, 10, dgamma_dbeta, C, 4, 1}, st)) return rc;
+    } else {
+        MMU_GN_DISPATCH((gn_bwd_reduce_kernel<TI, TO><<<rgrid, kGnThreads, smem, st>>>(
+            (const TI *)x, (const TO *)dy, mean, rstd, gamma, sums2, dgamma_dbeta, g)))
+        count_launch();
+    }
+    MMU_GN_DISPATCH((gn_bwd_apply_kernel<TI, TO><<<agrid, 256, 0, st>>>((const TI *)x, (const TO *)dy, mean, rstd, gamma, sums2, (TI *)dx, g)))
+    count_launch();
+    return check_launch("group_norm_nhwc_bwd");
+}
+}  // namespace
+}  // namespace mmu
+
+extern "C" int mmu_group_norm_nhwc_fwd(const void *x, const float *gamma, const float *beta, void *y, float *sums, float *mean, float *rstd,
+                                       int32_t in_dtype, int32_t out_dtype, int32_t B, int32_t C, int32_t HW, int32_t G, float eps, void *stream) {
+    return mmu::gn_fwd(x, gamma, beta, y, sums, mean, rstd, in_dtype, out_dtype, B, C, HW, G, eps, nullptr, static_cast<cudaStream_t>(stream));
 }
 
 // dy has dtype out_dtype (the forward's output dtype), dx has in_dtype.  sums2 (B*G*2) and dgamma_dbeta (2*C) are accumulated
@@ -229,15 +300,30 @@ extern "C" int mmu_group_norm_nhwc_fwd(const void *x, const float *gamma, const 
 extern "C" int mmu_group_norm_nhwc_bwd(const void *x, const float *gamma, const void *dy, const float *mean, const float *rstd, void *dx,
                                        float *sums2, float *dgamma_dbeta, int32_t in_dtype, int32_t out_dtype, int32_t B, int32_t C, int32_t HW,
                                        int32_t G, void *stream) {
+    return mmu::gn_bwd(x, gamma, dy, mean, rstd, dx, sums2, dgamma_dbeta, in_dtype, out_dtype, B, C, HW, G, nullptr,
+                       static_cast<cudaStream_t>(stream));
+}
+
+extern "C" size_t mmu_group_norm_nhwc_fwd_det_workspace(int32_t B, int32_t C, int32_t HW, int32_t G) { return mmu::gn_det_bytes(B, C, HW, G, 2); }
+extern "C" size_t mmu_group_norm_nhwc_bwd_det_workspace(int32_t B, int32_t C, int32_t HW, int32_t G) { return mmu::gn_det_bytes(B, C, HW, G, 10); }
+
+extern "C" int mmu_group_norm_nhwc_fwd_det(const void *x, const float *gamma, const float *beta, void *y, float *sums, float *mean, float *rstd,
+                                           int32_t in_dtype, int32_t out_dtype, int32_t B, int32_t C, int32_t HW, int32_t G, float eps, void *ws,
+                                           size_t ws_bytes, void *stream) {
     using namespace mmu;
-    GnGeom g;
-    dim3 rgrid, agrid;
-    if (int rc = gn_geom(g, B, C, HW, G, 0.f, rgrid, agrid)) return rc;
-    if (!x || !gamma || !dy || !mean || !rstd || !dx || !sums2 || !dgamma_dbeta) return set_error(MMU_ERR_INVALID, "group_norm_bwd: null pointer");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    MMU_GN_DISPATCH((gn_bwd_reduce_kernel<TI, TO><<<rgrid, kGnThreads, 10 * kGnThreads * sizeof(float), st>>>(
-        (const TI *)x, (const TO *)dy, mean, rstd, gamma, sums2, dgamma_dbeta, g)))
-    MMU_GN_DISPATCH((gn_bwd_apply_kernel<TI, TO><<<agrid, 256, 0, st>>>((const TI *)x, (const TO *)dy, mean, rstd, gamma, sums2, (TI *)dx, g)))
-    count_launch(2);
-    return check_launch("group_norm_nhwc_bwd");
+    const size_t need = mmu_group_norm_nhwc_fwd_det_workspace(B, C, HW, G);
+    if (need == 0) return set_error(MMU_ERR_INVALID, "group_norm_fwd_det: bad shape B%d C%d HW%d G%d", B, C, HW, G);
+    if (int rc = det_ws_check(ws, ws_bytes, need, "group_norm_nhwc_fwd_det")) return rc;
+    return gn_fwd(x, gamma, beta, y, sums, mean, rstd, in_dtype, out_dtype, B, C, HW, G, eps, static_cast<float *>(ws), static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int mmu_group_norm_nhwc_bwd_det(const void *x, const float *gamma, const void *dy, const float *mean, const float *rstd, void *dx,
+                                           float *sums2, float *dgamma_dbeta, int32_t in_dtype, int32_t out_dtype, int32_t B, int32_t C,
+                                           int32_t HW, int32_t G, void *ws, size_t ws_bytes, void *stream) {
+    using namespace mmu;
+    const size_t need = mmu_group_norm_nhwc_bwd_det_workspace(B, C, HW, G);
+    if (need == 0) return set_error(MMU_ERR_INVALID, "group_norm_bwd_det: bad shape B%d C%d HW%d G%d", B, C, HW, G);
+    if (int rc = det_ws_check(ws, ws_bytes, need, "group_norm_nhwc_bwd_det")) return rc;
+    return gn_bwd(x, gamma, dy, mean, rstd, dx, sums2, dgamma_dbeta, in_dtype, out_dtype, B, C, HW, G, static_cast<float *>(ws),
+                  static_cast<cudaStream_t>(stream));
 }

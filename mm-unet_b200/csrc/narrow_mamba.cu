@@ -51,6 +51,7 @@ struct NarArgs {
     float scope;
     const float *altho, *dcoords;
     float *coords;
+    float *part;             // deterministic backward: per (batch, tile) slots of the weight-gradient sums (NarDet)
 };
 
 __device__ __forceinline__ float coord_gain(float altho, float *dgain_daltho = nullptr) {
@@ -196,8 +197,8 @@ template <typename IN_T, typename HID_T, int DM> __global__ void __launch_bounds
     for (int e = 0; e < DM; ++e) op[(int64_t)e * p.o_cs] = Elem<IN_T>::from_f(v[e]);
 }
 
-// sum of v[i] over the block -> one atomicAdd per i
-template <int NV> __device__ __forceinline__ void block_sum_atomic(float (&v)[NV], float *dst, float *s_red /* [kNarT/32][NV] */) {
+// sum of v[i] over the block -> one atomicAdd per i (DET: one plain store per i into the block's own slot)
+template <int NV, bool DET> __device__ __forceinline__ void block_sum(float (&v)[NV], float *dst, float *s_red /* [kNarT/32][NV] */) {
 #pragma unroll
     for (int i = 0; i < NV; ++i) {
         float x = v[i];
@@ -210,11 +211,18 @@ template <int NV> __device__ __forceinline__ void block_sum_atomic(float (&v)[NV
         float x = 0.f;
 #pragma unroll
         for (int w = 0; w < kNarT / 32; ++w) x += s_red[w * NV + threadIdx.x];
-        atomicAdd(dst + threadIdx.x, x);
+        if constexpr (DET) dst[threadIdx.x] = x;
+        else atomicAdd(dst + threadIdx.x, x);
     }
 }
 
-template <typename IN_T, int DM> __global__ void __launch_bounds__(kNarT) narrow_post_bwd_kernel(const __grid_constant__ NarArgs p) {
+// Deterministic backward: the (batch, tile) work item's sums go to slot b * gridDim.x + tile of p.part - post_bwd: the out_proj | altho
+// floats [oWout, kNW], pre_bwd: every float below oWout - and the ordered reduce adds the slots into dweights.
+template <int DM> struct NarDet {
+    static constexpr int kPost = DM * Nar<DM>::DI + 1, kPre = Nar<DM>::oWout;
+};
+
+template <typename IN_T, int DM, bool DET = false> __global__ void __launch_bounds__(kNarT) narrow_post_bwd_kernel(const __grid_constant__ NarArgs p) {
     using C = Nar<DM>;
     __shared__ float s_wo[DM * C::DI];
     __shared__ float s_red[(kNarT / 32) * (DM * C::DI + 1)];
@@ -261,10 +269,11 @@ template <typename IN_T, int DM> __global__ void __launch_bounds__(kNarT) narrow
             for (int e = 0; e < DM; ++e) dw[e * C::DI + d] = g[e] * y[d];
         }
     }
-    block_sum_atomic<DM * C::DI + 1>(dw, p.dW + C::oWout, s_red);       // slot kNW = d(altho)
+    block_sum<DM * C::DI + 1, DET>(dw, DET ? p.part + ((int64_t)b * gridDim.x + blockIdx.x) * NarDet<DM>::kPost : p.dW + C::oWout,
+                                   s_red);       // slot kNW = d(altho)
 }
 
-template <typename IN_T, typename HID_T, int DM> __global__ void __launch_bounds__(kNarT) narrow_pre_bwd_kernel(const __grid_constant__ NarArgs p) {
+template <typename IN_T, typename HID_T, int DM, bool DET = false> __global__ void __launch_bounds__(kNarT) narrow_pre_bwd_kernel(const __grid_constant__ NarArgs p) {
     using C = Nar<DM>;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float *s_w = reinterpret_cast<float *>(smem_raw);                 // [kNW]
@@ -375,7 +384,8 @@ template <typename IN_T, typename HID_T, int DM> __global__ void __launch_bounds
         }
     }
     // conv weight / bias gradients: block sum of the per-token partials
-    block_sum_atomic<C::DI * 5>(cw, p.dW + C::oWc, s_red);       // conv_w (DI*4) and conv_b (DI) are adjacent in the weight block
+    float *dW = DET ? p.part + ((int64_t)b * gridDim.x + blockIdx.x) * NarDet<DM>::kPre : p.dW;
+    block_sum<C::DI * 5, DET>(cw, dW + C::oWc, s_red);       // conv_w (DI*4) and conv_b (DI) are adjacent in the weight block
     __syncthreads();
 
     // (3) x_proj / dt_proj / in_proj weight gradients: accumulator j = sum over the tile of rec[a_j] * rec[b_j]
@@ -397,7 +407,8 @@ template <typename IN_T, typename HID_T, int DM> __global__ void __launch_bounds
             acc1 = fmaf(s_rec[(t + 1) * C::kRec + a], s_rec[(t + 1) * C::kRec + bb], acc1);
         }
         if (t < ntok) acc0 = fmaf(s_rec[t * C::kRec + a], s_rec[t * C::kRec + bb], acc0);
-        atomicAdd(p.dW + dst, acc0 + acc1);
+        if constexpr (DET) dW[dst] = acc0 + acc1;
+        else atomicAdd(p.dW + dst, acc0 + acc1);
     }
 }
 
@@ -411,6 +422,21 @@ enum NarKernel { kPreFwd, kPostFwd, kPostBwd, kPreBwd };
 template <typename IN_T, typename HID_T> int launch_narrow(const NarArgs &a, NarKernel which, cudaStream_t st) {
     constexpr int DM = 3;
     dim3 grid((a.L + kNarT - 1) / kNarT, a.B);
+    if (a.part != nullptr) {
+        const int64_t items = (int64_t)a.B * grid.x;
+        if (which == kPostBwd) {
+            narrow_post_bwd_kernel<IN_T, DM, true><<<grid, kNarT, 0, st>>>(a);
+        } else {
+            auto k = narrow_pre_bwd_kernel<IN_T, HID_T, DM, true>;
+            constexpr size_t smem = pre_bwd_smem<DM>();
+            cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            k<<<grid, kNarT, smem, st>>>(a);
+        }
+        count_launch();
+        if (int rc = check_launch("mamba_narrow(deterministic)")) return rc;
+        const int nv = which == kPostBwd ? NarDet<DM>::kPost : NarDet<DM>::kPre;
+        return det_reduce(DetSum{a.part, items, nv, 1, 1, nv, 0, 0, a.dW + (which == kPostBwd ? Nar<DM>::oWout : 0), 0, 0, 1}, st);
+    }
     switch (which) {
         case kPreFwd: narrow_pre_fwd_kernel<IN_T, HID_T, DM><<<grid, kNarT, 0, st>>>(a); break;
         case kPostFwd: narrow_post_fwd_kernel<IN_T, HID_T, DM><<<grid, kNarT, 0, st>>>(a); break;
@@ -427,7 +453,7 @@ template <typename IN_T, typename HID_T> int launch_narrow(const NarArgs &a, Nar
     return check_launch("mamba_narrow");
 }
 
-int narrow_entry(const mmu_narrow_params *p, NarKernel which, void *stream) {
+int narrow_entry(const mmu_narrow_params *p, NarKernel which, float *part, void *stream) {
     if (p == nullptr) return set_error(MMU_ERR_INVALID, "mamba_narrow: null params");
     if (!mmu_mamba_narrow_supported(p->d_model, p->d_inner, p->d_state, p->dt_rank, p->d_conv, p->dtype))
         return set_error(MMU_ERR_UNSUPPORTED, "mamba_narrow: d_model %d d_inner %d d_state %d dt_rank %d d_conv %d dtype %d is not a narrow block",
@@ -440,6 +466,7 @@ int narrow_entry(const mmu_narrow_params *p, NarKernel which, void *stream) {
     a.h_bs = p->hidden_bs, a.h_cs = p->hidden_cs, a.o_bs = p->out_bs, a.o_cs = p->out_cs;
     a.g_bs = p->dout_bs, a.g_cs = p->dout_cs, a.dh_bs = p->dhidden_bs, a.dh_cs = p->dhidden_cs;
     a.B = p->batch, a.L = p->seqlen;
+    a.part = part;
     if (!make_ordmap(a.ord, p->order, p->order_h, p->order_w, p->order_ns, p->seqlen) || p->order == MMU_ORDER_FLIP)
         return set_error(MMU_ERR_INVALID, "mamba_narrow: bad scan order %d (H=%d W=%d nslices=%d, L=%d)", p->order, p->order_h, p->order_w,
                          p->order_ns, p->seqlen);
@@ -473,7 +500,40 @@ extern "C" int32_t mmu_mamba_narrow_rows(int32_t d_inner, int32_t d_state) { ret
 extern "C" int32_t mmu_mamba_narrow_weight_floats(int32_t d_model, int32_t d_inner, int32_t d_state, int32_t dt_rank, int32_t d_conv) {
     return 2 * d_inner * d_model + d_inner * d_conv + d_inner + (dt_rank + 2 * d_state) * d_inner + d_inner * dt_rank + d_model * d_inner + 1;
 }
-extern "C" int mmu_mamba_narrow_pre_fwd(const mmu_narrow_params *p, void *stream) { return mmu::narrow_entry(p, mmu::kPreFwd, stream); }
-extern "C" int mmu_mamba_narrow_post_fwd(const mmu_narrow_params *p, void *stream) { return mmu::narrow_entry(p, mmu::kPostFwd, stream); }
-extern "C" int mmu_mamba_narrow_post_bwd(const mmu_narrow_params *p, void *stream) { return mmu::narrow_entry(p, mmu::kPostBwd, stream); }
-extern "C" int mmu_mamba_narrow_pre_bwd(const mmu_narrow_params *p, void *stream) { return mmu::narrow_entry(p, mmu::kPreBwd, stream); }
+extern "C" int mmu_mamba_narrow_pre_fwd(const mmu_narrow_params *p, void *stream) { return mmu::narrow_entry(p, mmu::kPreFwd, nullptr, stream); }
+extern "C" int mmu_mamba_narrow_post_fwd(const mmu_narrow_params *p, void *stream) { return mmu::narrow_entry(p, mmu::kPostFwd, nullptr, stream); }
+extern "C" int mmu_mamba_narrow_post_bwd(const mmu_narrow_params *p, void *stream) { return mmu::narrow_entry(p, mmu::kPostBwd, nullptr, stream); }
+extern "C" int mmu_mamba_narrow_pre_bwd(const mmu_narrow_params *p, void *stream) { return mmu::narrow_entry(p, mmu::kPreBwd, nullptr, stream); }
+
+namespace mmu {
+namespace {
+size_t narrow_det_bytes(int32_t batch, int32_t seqlen, int per_tile) {
+    if (batch <= 0 || seqlen <= 0) return 0;
+    DetWs w{nullptr};
+    w.take((size_t)batch * ((seqlen + kNarT - 1) / kNarT) * per_tile);
+    return w.used;
+}
+int narrow_det(const mmu_narrow_params *p, NarKernel which, void *ws, size_t ws_bytes, void *stream) {
+    const char *what = which == kPostBwd ? "mamba_narrow_post_bwd_det" : "mamba_narrow_pre_bwd_det";
+    if (p == nullptr) return set_error(MMU_ERR_INVALID, "%s: null params", what);
+    const size_t need = which == kPostBwd ? mmu_mamba_narrow_post_bwd_det_workspace(p->batch, p->seqlen)
+                                          : mmu_mamba_narrow_pre_bwd_det_workspace(p->batch, p->seqlen);
+    if (need == 0) return set_error(MMU_ERR_INVALID, "%s: bad shape", what);
+    if (int rc = det_ws_check(ws, ws_bytes, need, what)) return rc;
+    return narrow_entry(p, which, static_cast<float *>(ws), stream);
+}
+}  // namespace
+}  // namespace mmu
+
+extern "C" size_t mmu_mamba_narrow_post_bwd_det_workspace(int32_t batch, int32_t seqlen) {
+    return mmu::narrow_det_bytes(batch, seqlen, mmu::NarDet<3>::kPost);
+}
+extern "C" size_t mmu_mamba_narrow_pre_bwd_det_workspace(int32_t batch, int32_t seqlen) {
+    return mmu::narrow_det_bytes(batch, seqlen, mmu::NarDet<3>::kPre);
+}
+extern "C" int mmu_mamba_narrow_post_bwd_det(const mmu_narrow_params *p, void *ws, size_t ws_bytes, void *stream) {
+    return mmu::narrow_det(p, mmu::kPostBwd, ws, ws_bytes, stream);
+}
+extern "C" int mmu_mamba_narrow_pre_bwd_det(const mmu_narrow_params *p, void *ws, size_t ws_bytes, void *stream) {
+    return mmu::narrow_det(p, mmu::kPreBwd, ws, ws_bytes, stream);
+}

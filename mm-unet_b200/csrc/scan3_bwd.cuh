@@ -32,6 +32,7 @@ struct Bwd3Args {
     int nseg, cps, nchunks, nx;
     int softplus;
     OrdMap ord;                    // ORD kernels: z, dout and dz live at ord(l) (natural token order), everything else at l
+    int64_t det_rgs;               // DET kernels: row-group stride of the dB / dC slots (dB, dC point at the slots)
 #if MMU_TMA_TILE
     alignas(64) unsigned char tmB[128], tmC[128];   // CUtensorMap of B and C (see Fwd3Args)
 #endif
@@ -59,7 +60,10 @@ __device__ __forceinline__ void red_add_v4(float *p, float a, float b, float c, 
 
 // ORD: fused scan order (NSLICES / TWOROW): z and dout are gathered, dz is scattered through p.ord (ord_issue8 / ord_store8 in
 // scan3.cuh); never together with REV.
-template <typename IN_T, int W, bool REV, bool AGG, bool ORD = false>
+// DET (deterministic mode, main pass only): no float atomics.  dB / dC / dA / dD / ddbias point at slots of the caller's workspace:
+// the CTA STORES its slab sums to dB / dC + row group * det_rgs (each (row group, batch, state, token) has exactly one writer), and
+// dA / dD / ddbias to [batch][segment][row](x dstate).  The ordered reduce (det_reduce.cu) adds the slots to the real outputs.
+template <typename IN_T, int W, bool REV, bool AGG, bool ORD = false, bool DET = false>
 __global__ void __launch_bounds__(32 * W, AGG ? 1 : 8 / W) scan3_bwd_kernel(const __grid_constant__ Bwd3Args p) {
     static_assert(!ORD || !REV, "ordered gate / output gradient: forward direction only");
     using Cfg = Bwd3Cfg<IN_T, W>;
@@ -169,8 +173,8 @@ __global__ void __launch_bounds__(32 * W, AGG ? 1 : 8 / W) scan3_bwd_kernel(cons
     [[maybe_unused]] int tin = tl + CH;      // ORD: first logical token of my 8 in the chunk being prefetched (one step behind, like the pointers)
     const IN_T *B_b = reinterpret_cast<const IN_T *>(p.Bm) + (int64_t)b * p.B_bs;
     const IN_T *C_b = reinterpret_cast<const IN_T *>(p.Cm) + (int64_t)b * p.C_bs;
-    float *dB_b = AGG ? nullptr : p.dB + (int64_t)b * p.dB_bs;
-    float *dC_b = AGG ? nullptr : p.dC + (int64_t)b * p.dC_bs;
+    float *dB_b = AGG ? nullptr : p.dB + (int64_t)b * p.dB_bs + (DET ? (int64_t)bx * p.det_rgs : 0);
+    float *dC_b = AGG ? nullptr : p.dC + (int64_t)b * p.dC_bs + (DET ? (int64_t)bx * p.det_rgs : 0);
 
     bool ge_up[3], ge_dn[5];
 #pragma unroll
@@ -493,7 +497,8 @@ __global__ void __launch_bounds__(32 * W, AGG ? 1 : 8 / W) scan3_bwd_kernel(cons
                     const int tq = t0c + 8 * l + 4 * q;
                     if (tq < L) {
                         float *dst = (which ? dC_b + (int64_t)n * p.dC_ns : dB_b + (int64_t)n * p.dB_ns) + (REV ? L - 4 - tq : tq);
-                        if (REV) red_add_v4(dst, v.w, v.z, v.y, v.x);
+                        if constexpr (DET) *reinterpret_cast<float4 *>(dst) = REV ? make_float4(v.w, v.z, v.y, v.x) : v;
+                        else if (REV) red_add_v4(dst, v.w, v.z, v.y, v.x);
                         else red_add_v4(dst, v.x, v.y, v.z, v.w);
                     }
                 }
@@ -613,8 +618,14 @@ __global__ void __launch_bounds__(32 * W, AGG ? 1 : 8 / W) scan3_bwd_kernel(cons
                 v.y += __shfl_xor_sync(0xffffffffu, v.y, k);
             }
             if (j == 0) {
-                if (row_ok[0]) atomicAdd(p.dA + (int64_t)rowA * N + n, v.x);
-                if (row_ok[1]) atomicAdd(p.dA + (int64_t)(rowA + 1) * N + n, v.y);
+                if constexpr (DET) {
+                    float *slot = p.dA + ((int64_t)b * p.nseg + seg) * D * N;
+                    if (row_ok[0]) slot[(int64_t)rowA * N + n] = v.x;
+                    if (row_ok[1]) slot[(int64_t)(rowA + 1) * N + n] = v.y;
+                } else {
+                    if (row_ok[0]) atomicAdd(p.dA + (int64_t)rowA * N + n, v.x);
+                    if (row_ok[1]) atomicAdd(p.dA + (int64_t)(rowA + 1) * N + n, v.y);
+                }
             }
         }
         float2 dd = dDacc, db = dbacc;
@@ -627,8 +638,14 @@ __global__ void __launch_bounds__(32 * W, AGG ? 1 : 8 / W) scan3_bwd_kernel(cons
 #pragma unroll
             for (int r = 0; r < 2; ++r) {
                 if (row_ok[r]) {
-                    if (p.dD != nullptr) atomicAdd(p.dD + rowA + r, r ? dd.y : dd.x);
-                    if (p.ddbias != nullptr) atomicAdd(p.ddbias + rowA + r, r ? db.y : db.x);
+                    if constexpr (DET) {
+                        const int64_t slot = ((int64_t)b * p.nseg + seg) * D + rowA + r;
+                        if (p.dD != nullptr) p.dD[slot] = r ? dd.y : dd.x;
+                        if (p.ddbias != nullptr) p.ddbias[slot] = r ? db.y : db.x;
+                    } else {
+                        if (p.dD != nullptr) atomicAdd(p.dD + rowA + r, r ? dd.y : dd.x);
+                        if (p.ddbias != nullptr) atomicAdd(p.ddbias + rowA + r, r ? db.y : db.x);
+                    }
                 }
             }
         }

@@ -38,6 +38,7 @@ struct BwdArgs {
     int nseg, cps, nchunks, nx;
     int softplus, reverse;
     unsigned vec_mask;   // bit0 u, 1 delta, 2 z, 3 dout, 4 B, 5 C, 6 du, 7 ddelta, 8 dz
+    int64_t det_rgs;     // DET kernels: row-group stride of the dB / dC slots
 };
 
 template <int RQ, int NGW> struct BwdCfg {
@@ -50,7 +51,9 @@ template <int RQ, int NGW> struct BwdCfg {
     }
 };
 
-template <typename IN_T, int RQ, int NGW, bool AGG, int MINB>
+// DET (deterministic mode, main pass only): as scan3_bwd_kernel's DET - dB / dC / dA / dD / ddbias point at the caller's slots, the
+// CTA stores its sums there, and dD / ddbias are summed over the CTA in a fixed order instead of with shared-memory atomics.
+template <typename IN_T, int RQ, int NGW, bool AGG, int MINB, bool DET = false>
 __global__ void __launch_bounds__(32 * RQ * NGW, AGG ? 512 / (32 * RQ * NGW) : MINB) scan_bwd_kernel(const __grid_constant__ BwdArgs p) {
     using Cfg = BwdCfg<RQ, NGW>;
     constexpr int T = Cfg::T, R = Cfg::R, TL = Cfg::TL, NT = Cfg::NT, NW = Cfg::NW;
@@ -421,7 +424,8 @@ __global__ void __launch_bounds__(32 * RQ * NGW, AGG ? 512 / (32 * RQ * NGW) : M
         }
         // ---- epilogue B: dB / dC -> global (sum over the CTA's row-warps, then one atomic per element) ---------------
         {
-            float *dB_b = p.dB + (int64_t)b * p.dB_bs, *dC_b = p.dC + (int64_t)b * p.dC_bs;
+            float *dB_b = p.dB + (int64_t)b * p.dB_bs + (DET ? (int64_t)blockIdx.x * p.det_rgs : 0);
+            float *dC_b = p.dC + (int64_t)b * p.dC_bs + (DET ? (int64_t)blockIdx.x * p.det_rgs : 0);
             for (int idx = tid; idx < NP * TL; idx += NT) {
                 const int tok = idx % TL, pr = idx / TL;
                 const int e = ((tok & 7) << 3) | (tok >> 3);            // staging order: e = 8*i + j for token 8*j + i
@@ -435,11 +439,20 @@ __global__ void __launch_bounds__(32 * RQ * NGW, AGG ? 512 / (32 * RQ * NGW) : M
                 const int t = t0 + tok, n0 = 2 * pr;
                 if (t < L) {
                     const int64_t m = rev ? L - 1 - t : t;
-                    atomicAdd(dB_b + (int64_t)n0 * p.dB_ns + m, v.x);
-                    atomicAdd(dC_b + (int64_t)n0 * p.dC_ns + m, v.z);
-                    if (n0 + 1 < N) {
-                        atomicAdd(dB_b + (int64_t)(n0 + 1) * p.dB_ns + m, v.y);
-                        atomicAdd(dC_b + (int64_t)(n0 + 1) * p.dC_ns + m, v.w);
+                    if constexpr (DET) {
+                        dB_b[(int64_t)n0 * p.dB_ns + m] = v.x;
+                        dC_b[(int64_t)n0 * p.dC_ns + m] = v.z;
+                        if (n0 + 1 < N) {
+                            dB_b[(int64_t)(n0 + 1) * p.dB_ns + m] = v.y;
+                            dC_b[(int64_t)(n0 + 1) * p.dC_ns + m] = v.w;
+                        }
+                    } else {
+                        atomicAdd(dB_b + (int64_t)n0 * p.dB_ns + m, v.x);
+                        atomicAdd(dC_b + (int64_t)n0 * p.dC_ns + m, v.z);
+                        if (n0 + 1 < N) {
+                            atomicAdd(dB_b + (int64_t)(n0 + 1) * p.dB_ns + m, v.y);
+                            atomicAdd(dC_b + (int64_t)(n0 + 1) * p.dC_ns + m, v.w);
+                        }
                     }
                 }
             }
@@ -471,8 +484,28 @@ __global__ void __launch_bounds__(32 * RQ * NGW, AGG ? 512 / (32 * RQ * NGW) : M
                 float v = 0.f;
 #pragma unroll
                 for (int k = 0; k < 8; ++k) v += src[2 * k];
-                atomicAdd(p.dA + (int64_t)row * N + n, v);           // sum over batch and segments
+                if constexpr (DET) p.dA[((int64_t)b * p.nseg + seg) * D * N + (int64_t)row * N + n] = v;
+                else atomicAdd(p.dA + (int64_t)row * N + n, v);           // sum over batch and segments
             }
+        }
+        if constexpr (DET) {      // dD / ddelta_bias: the row's TL/4 quad partials (s_part is free now), summed in quad order
+#pragma unroll
+            for (int k = 0; k < KR; ++k) {
+                const int idx = tid + k * NT;
+                if (idx < QT) s_part[idx] = acc_dD[k], s_part[QT + idx] = acc_db[k];
+            }
+            __syncthreads();
+            for (int r = tid; r < R; r += NT) {
+                const int row = row0 + r;
+                if (row < D) {
+                    float sd = 0.f, sb = 0.f;
+                    for (int q = 0; q < TL / 4; ++q) sd += s_part[r * (TL / 4) + q], sb += s_part[QT + r * (TL / 4) + q];
+                    const int64_t slot = ((int64_t)b * p.nseg + seg) * D + row;
+                    if (p.dD != nullptr) p.dD[slot] = sd;
+                    if (p.ddbias != nullptr) p.ddbias[slot] = sb;
+                }
+            }
+            return;
         }
 #pragma unroll
         for (int k = 0; k < KR; ++k) {
@@ -545,12 +578,16 @@ BwdPlan plan_bwd(int B, int D, int L) {
     return pl;
 }
 
-template <typename IN_T, int RQ, int NGW, int MINB> int launch_bwd(const BwdArgs &a, bool agg, cudaStream_t st) {
+template <typename IN_T, int RQ, int NGW, int MINB> int launch_bwd(const BwdArgs &a, bool agg, bool det, cudaStream_t st) {
     using Cfg = BwdCfg<RQ, NGW>;
     const size_t smem = Cfg::smem_floats(a.Ne) * sizeof(float);
     if (smem > 227 * 1024) return set_error(MMU_ERR_UNSUPPORTED, "selective_scan_bwd: dstate %d needs %zu B smem", a.N, smem);
     dim3 grid((a.D + Cfg::R - 1) / Cfg::R, a.B, a.nseg), block(Cfg::NT);
-    if (agg) {
+    if (det && !agg) {
+        auto k = scan_bwd_kernel<IN_T, RQ, NGW, false, MINB, true>;
+        cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        k<<<grid, block, smem, st>>>(a);
+    } else if (agg) {
         auto k = scan_bwd_kernel<IN_T, RQ, NGW, true, MINB>;
         cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         k<<<grid, block, smem, st>>>(a);
@@ -563,14 +600,56 @@ template <typename IN_T, int RQ, int NGW, int MINB> int launch_bwd(const BwdArgs
     return check_launch("selective_scan_bwd");
 }
 
-template <typename IN_T> int dispatch_bwd(int cfg, const BwdArgs &a, bool agg, cudaStream_t st) {
+template <typename IN_T> int dispatch_bwd(int cfg, const BwdArgs &a, bool agg, cudaStream_t st, bool det = false) {
     switch (cfg) {
-        case 0: return launch_bwd<IN_T, 2, 2, 3>(a, agg, st);
-        case 1: return launch_bwd<IN_T, 1, 4, 3>(a, agg, st);
-        case 2: return launch_bwd<IN_T, 2, 4, 1>(a, agg, st);
-        case 3: return launch_bwd<IN_T, 2, 2, 2>(a, agg, st);
-        default: return launch_bwd<IN_T, 2, 2, 4>(a, agg, st);
+        case 0: return launch_bwd<IN_T, 2, 2, 3>(a, agg, det, st);
+        case 1: return launch_bwd<IN_T, 1, 4, 3>(a, agg, det, st);
+        case 2: return launch_bwd<IN_T, 2, 4, 1>(a, agg, det, st);
+        case 3: return launch_bwd<IN_T, 2, 2, 2>(a, agg, det, st);
+        default: return launch_bwd<IN_T, 2, 2, 4>(a, agg, det, st);
     }
+}
+
+// ---- deterministic mode: partial slots in the caller's workspace, then ordered reduces -----------------------------------------
+// Slot layout (fixed for a shape, whichever kernel runs): dB and dC [row group][batch][dstate][seqlen], dA [batch][segment][dim][dstate],
+// dD and ddelta_bias [batch][segment][dim], each sized for the most row groups / segments any plan of this shape can use.
+struct ScanDet {
+    float *pB, *pC, *pA, *pD, *pdb;
+};
+struct ScanDetBound {
+    int64_t nrg, nseg;
+};
+ScanDetBound scan_det_bound(int B, int D, int L);   // below the plans
+size_t scan_det_carve(int B, int D, int L, int N, char *base, ScanDet *d) {
+    const ScanDetBound bd = scan_det_bound(B, D, L);
+    DetWs w{base};
+    const size_t bc = (size_t)bd.nrg * B * N * L, a = (size_t)B * bd.nseg * D * N, r = (size_t)B * bd.nseg * D;
+    ScanDet t{w.take(bc), w.take(bc), w.take(a), w.take(r), w.take(r)};
+    if (d != nullptr) *d = t;
+    return w.used;
+}
+// point the kernel's gradient outputs at the slots
+template <typename Args> void scan_det_args(Args &a, const ScanDet &d) {
+    a.dB = d.pB, a.dC = d.pC, a.dA = d.pA;
+    a.dD = a.dD ? d.pD : nullptr, a.ddbias = a.ddbias ? d.pdb : nullptr;
+    a.dB_bs = a.dC_bs = (int64_t)a.N * a.L, a.dB_ns = a.dC_ns = a.L;
+    a.det_rgs = (int64_t)a.B * a.N * a.L;
+}
+// sum the slots of the nrg row groups / nseg segments the kernel used into the caller's outputs
+int scan_det_reduce(const mmu_scan_bwd_params *p, const ScanDet &d, int nrg, int nseg, cudaStream_t st) {
+    const mmu_scan_fwd_params &f = p->f;
+    const int B = f.batch, D = f.dim, L = f.seqlen, N = f.dstate;
+    const int64_t dB_bs = p->dB_bs ? p->dB_bs : (int64_t)N * L, dC_bs = p->dC_bs ? p->dC_bs : (int64_t)N * L;
+    const int64_t dB_ns = p->dB_ns ? p->dB_ns : L, dC_ns = p->dC_ns ? p->dC_ns : L;
+    const int64_t rgs = (int64_t)B * N * L, items = (int64_t)B * nseg;
+    if (int rc = det_reduce(DetSum{d.pB, nrg, rgs, B, N, L, (int64_t)N * L, L, p->dB, dB_bs, dB_ns, 1}, st)) return rc;
+    if (int rc = det_reduce(DetSum{d.pC, nrg, rgs, B, N, L, (int64_t)N * L, L, p->dC, dC_bs, dC_ns, 1}, st)) return rc;
+    if (int rc = det_reduce(DetSum{d.pA, items, (int64_t)D * N, 1, 1, D * N, 0, 0, p->dA, 0, 0, 1}, st)) return rc;
+    if (p->dD != nullptr)
+        if (int rc = det_reduce(DetSum{d.pD, items, D, 1, 1, D, 0, 0, p->dD, 0, 0, 1}, st)) return rc;
+    if (p->ddelta_bias != nullptr)
+        if (int rc = det_reduce(DetSum{d.pdb, items, D, 1, 1, D, 0, 0, p->ddelta_bias, 0, 0, 1}, st)) return rc;
+    return MMU_OK;
 }
 
 // ---- v3 host side (scan3_bwd.cuh) ------------------------------------------------------------------------------------------
@@ -631,10 +710,10 @@ Bwd3Plan plan_bwd3(int B, int D, int L, bool ordered = false) {
     return pl;
 }
 
-template <typename IN_T, int W, bool REV, bool AGG, bool ORD = false> int launch_bwd3(const Bwd3Args &a, cudaStream_t st) {
+template <typename IN_T, int W, bool REV, bool AGG, bool ORD = false, bool DET = false> int launch_bwd3(const Bwd3Args &a, cudaStream_t st) {
     using Cfg = Bwd3Cfg<IN_T, W>;
     dim3 grid((a.D + Cfg::R - 1) / Cfg::R, a.B, a.nseg), block(Cfg::NT);
-    auto k = scan3_bwd_kernel<IN_T, W, REV, AGG, ORD>;
+    auto k = scan3_bwd_kernel<IN_T, W, REV, AGG, ORD, DET>;
     const size_t smem = Cfg::smem_bytes;
     cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     k<<<grid, block, smem, st>>>(a);
@@ -642,14 +721,14 @@ template <typename IN_T, int W, bool REV, bool AGG, bool ORD = false> int launch
     return check_launch("selective_scan_bwd(v3)");
 }
 
-template <typename IN_T, bool AGG> int dispatch_bwd3(const Bwd3Args &a, int W, bool rev, cudaStream_t st) {
+template <typename IN_T, bool AGG, bool DET = false> int dispatch_bwd3(const Bwd3Args &a, int W, bool rev, cudaStream_t st) {
     if (a.ord.kind != MMU_ORDER_ROWMAJOR) {         // fused scan order: z / dout / dz permuted by the kernel (never with rev)
-        if (W == 1) return launch_bwd3<IN_T, 1, false, AGG, true>(a, st);
-        if (W == 2) return launch_bwd3<IN_T, 2, false, AGG, true>(a, st);
-        if (W == 3) return launch_bwd3<IN_T, 3, false, AGG, true>(a, st);
-        return launch_bwd3<IN_T, 4, false, AGG, true>(a, st);
+        if (W == 1) return launch_bwd3<IN_T, 1, false, AGG, true, DET>(a, st);
+        if (W == 2) return launch_bwd3<IN_T, 2, false, AGG, true, DET>(a, st);
+        if (W == 3) return launch_bwd3<IN_T, 3, false, AGG, true, DET>(a, st);
+        return launch_bwd3<IN_T, 4, false, AGG, true, DET>(a, st);
     }
-#define MMU_B3(W_) (rev ? launch_bwd3<IN_T, W_, true, AGG>(a, st) : launch_bwd3<IN_T, W_, false, AGG>(a, st))
+#define MMU_B3(W_) (rev ? launch_bwd3<IN_T, W_, true, AGG, false, DET>(a, st) : launch_bwd3<IN_T, W_, false, AGG, false, DET>(a, st))
     if (W == 1) return MMU_B3(1);
     if (W == 2) return MMU_B3(2);
     if (W == 3) return MMU_B3(3);
@@ -658,7 +737,18 @@ template <typename IN_T, bool AGG> int dispatch_bwd3(const Bwd3Args &a, int W, b
 #undef MMU_B3
 }
 
-template <typename IN_T> int run_bwd3(const mmu_scan_bwd_params *p, cudaStream_t st) {
+// the main pass; det != nullptr: the DET kernels into the slots, then the ordered reduces
+template <typename IN_T> int run_bwd3_main(const Bwd3Args &a0, const mmu_scan_bwd_params *p, const Bwd3Plan &pl, const ScanDet *det,
+                                           cudaStream_t st) {
+    const bool rev = p->f.reverse != 0;
+    if (det == nullptr) return dispatch_bwd3<IN_T, false>(a0, pl.W, rev, st);
+    Bwd3Args a = a0;
+    scan_det_args(a, *det);
+    if (int rc = dispatch_bwd3<IN_T, false, true>(a, pl.W, rev, st)) return rc;
+    return scan_det_reduce(p, *det, (a.D + 2 * pl.W - 1) / (2 * pl.W), pl.nseg, st);
+}
+
+template <typename IN_T> int run_bwd3(const mmu_scan_bwd_params *p, cudaStream_t st, const ScanDet *det) {
     const mmu_scan_fwd_params &f = p->f;
     const Bwd3Plan pl = plan_bwd3(f.batch, f.dim, f.seqlen, f.order != MMU_ORDER_ROWMAJOR);
     Bwd3Args a{};
@@ -696,7 +786,7 @@ template <typename IN_T> int run_bwd3(const mmu_scan_bwd_params *p, cudaStream_t
         a.chain_flags = reinterpret_cast<int *>(w + align256(n_state * 4));
         a.chain_ticket = a.chain_flags + (n_flags - 1);
         cudaMemsetAsync(a.chain_flags, 0, n_flags * 4, st);
-        return dispatch_bwd3<IN_T, false>(a, pl.W, rev, st);
+        return run_bwd3_main<IN_T>(a, p, pl, det, st);
     }
     if (pl.nseg > 1) {
         const size_t n_state = (size_t)a.B * a.D * pl.nseg * 16, n_row = (size_t)a.B * a.D * pl.nseg;
@@ -717,7 +807,7 @@ template <typename IN_T> int run_bwd3(const mmu_scan_bwd_params *p, cudaStream_t
         if (rc) return rc;
         a.ein = ein;
     }
-    return dispatch_bwd3<IN_T, false>(a, pl.W, rev, st);
+    return run_bwd3_main<IN_T>(a, p, pl, det, st);
 }
 
 
@@ -811,7 +901,7 @@ template <typename IN_T> struct HasV3 { static constexpr bool value = false; };
 template <> struct HasV3<float> { static constexpr bool value = true; };
 template <> struct HasV3<__nv_bfloat16> { static constexpr bool value = true; };
 
-template <typename IN_T> int run_bwd(const mmu_scan_bwd_params *p, cudaStream_t st) {
+template <typename IN_T> int run_bwd(const mmu_scan_bwd_params *p, cudaStream_t st, const ScanDet *det) {
     if (p->f.order != MMU_ORDER_ROWMAJOR) {      // fused scan order: only on the dstate <= 16 kernels, only for the fusable maps
         const mmu_scan_fwd_params &f = p->f;
         bool ok = f.order != MMU_ORDER_FLIP && !f.reverse && ordmap_fusable(f.order, f.order_h, f.order_w, f.order_ns, f.seqlen) &&
@@ -821,16 +911,16 @@ template <typename IN_T> int run_bwd(const mmu_scan_bwd_params *p, cudaStream_t 
         if (!ok)
             return set_error(MMU_ERR_UNSUPPORTED, "selective_scan_bwd: scan order %d (H=%d W=%d nslices=%d) cannot be fused for this problem "
                              "(see mmu_scan_order_fusable)", f.order, f.order_h, f.order_w, f.order_ns);
-        if constexpr (HasV3<IN_T>::value) return run_bwd3<IN_T>(p, st);
+        if constexpr (HasV3<IN_T>::value) return run_bwd3<IN_T>(p, st, det);
     }
     if constexpr (HasV3<IN_T>::value) {
-        if (bwd4_eligible<IN_T>(p)) return run_bwd4<IN_T>(p, st);
+        if (det == nullptr && bwd4_eligible<IN_T>(p)) return run_bwd4<IN_T>(p, st);      // opt-in experiment: never deterministic
     }
     if (p->f.x_stride != 0 && p->f.x_stride != MMU_STATE_STRIDE)
         return set_error(MMU_ERR_UNSUPPORTED, "selective_scan_bwd: x_stride %d needs the wide (v4) kernels (dim >= 64, dstate <= 16, "
                          "seqlen %% 8 == 0, 16-byte aligned rows)", p->f.x_stride);
     if constexpr (HasV3<IN_T>::value) {
-        if (bwd3_eligible<IN_T>(p)) return run_bwd3<IN_T>(p, st);
+        if (bwd3_eligible<IN_T>(p)) return run_bwd3<IN_T>(p, st, det);
     }
     const mmu_scan_fwd_params &f = p->f;
     const BwdPlan pl = plan_bwd(f.batch, f.dim, f.seqlen);
@@ -883,7 +973,19 @@ template <typename IN_T> int run_bwd(const mmu_scan_bwd_params *p, cudaStream_t 
         if (rc) return rc;
         a.dhin = dhin;
     }
-    return dispatch_bwd<IN_T>(pl.cfg, a, false, st);
+    if (det == nullptr) return dispatch_bwd<IN_T>(pl.cfg, a, false, st);
+    scan_det_args(a, *det);
+    if (int rc = dispatch_bwd<IN_T>(pl.cfg, a, false, st, true)) return rc;
+    return scan_det_reduce(p, *det, (a.D + pl.R - 1) / pl.R, pl.nseg, st);
+}
+
+ScanDetBound scan_det_bound(int B, int D, int L) {
+    const Bwd3Plan a = plan_bwd3(B, D, L, false), o = plan_bwd3(B, D, L, true);
+    const BwdPlan v1 = plan_bwd(B, D, L);
+    ScanDetBound bd;
+    bd.nrg = std::max({(D + 2 * a.W - 1) / (2 * a.W), (D + 2 * o.W - 1) / (2 * o.W), (D + v1.R - 1) / v1.R});
+    bd.nseg = std::max({a.nseg, o.nseg, v1.nseg});
+    return bd;
 }
 
 }  // namespace
@@ -911,8 +1013,34 @@ extern "C" int32_t mmu_scan_state_stride(int32_t batch, int32_t dim, int32_t seq
     return v4 ? 8 : MMU_STATE_STRIDE;
 }
 
-extern "C" int mmu_selective_scan_bwd(const mmu_scan_bwd_params *p, void *stream) {
+namespace mmu {
+namespace {
+int scan_bwd_entry(const mmu_scan_bwd_params *p, const ScanDet *det, void *stream);
+}
+}  // namespace mmu
+
+extern "C" size_t mmu_selective_scan_bwd_det_workspace(int32_t batch, int32_t dim, int32_t seqlen, int32_t dstate) {
+    if (batch <= 0 || dim <= 0 || seqlen <= 0 || dstate <= 0) return 0;
+    return mmu::scan_det_carve(batch, dim, seqlen, dstate, nullptr, nullptr);
+}
+
+extern "C" int mmu_selective_scan_bwd_det(const mmu_scan_bwd_params *p, void *ws, size_t ws_bytes, void *stream) {
     using namespace mmu;
+    if (p == nullptr) return set_error(MMU_ERR_INVALID, "selective_scan_bwd_det: null params");
+    const mmu_scan_fwd_params &f = p->f;
+    const size_t need = mmu_selective_scan_bwd_det_workspace(f.batch, f.dim, f.seqlen, f.dstate);
+    if (need == 0) return set_error(MMU_ERR_INVALID, "selective_scan_bwd_det: empty shape");
+    if (int rc = det_ws_check(ws, ws_bytes, need, "selective_scan_bwd_det")) return rc;
+    ScanDet d;
+    scan_det_carve(f.batch, f.dim, f.seqlen, f.dstate, static_cast<char *>(ws), &d);
+    return scan_bwd_entry(p, &d, stream);
+}
+
+extern "C" int mmu_selective_scan_bwd(const mmu_scan_bwd_params *p, void *stream) { return mmu::scan_bwd_entry(p, nullptr, stream); }
+
+namespace mmu {
+namespace {
+int scan_bwd_entry(const mmu_scan_bwd_params *p, const ScanDet *det, void *stream) {
     if (p == nullptr) return set_error(MMU_ERR_INVALID, "selective_scan_bwd: null params");
     const mmu_scan_fwd_params &f = p->f;
     if (f.batch <= 0 || f.dim <= 0 || f.seqlen <= 0 || f.dstate <= 0)
@@ -927,9 +1055,11 @@ extern "C" int mmu_selective_scan_bwd(const mmu_scan_bwd_params *p, void *stream
         return set_error(MMU_ERR_INVALID, "selective_scan_bwd: dD / ddelta_bias missing");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     switch (f.dtype) {
-        case MMU_F32: return run_bwd<float>(p, st);
-        case MMU_BF16: return run_bwd<__nv_bfloat16>(p, st);
-        case MMU_F16: return run_bwd<__half>(p, st);
+        case MMU_F32: return run_bwd<float>(p, st, det);
+        case MMU_BF16: return run_bwd<__nv_bfloat16>(p, st, det);
+        case MMU_F16: return run_bwd<__half>(p, st, det);
         default: return set_error(MMU_ERR_UNSUPPORTED, "selective_scan_bwd: dtype %d", f.dtype);
     }
 }
+}  // namespace
+}  // namespace mmu

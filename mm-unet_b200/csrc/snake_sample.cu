@@ -12,6 +12,7 @@
 // map, output written directly in the consumer's dtype.
 // Backward: d_feat (fp32, caller zero-fills) receives the two taps by red.global.add.f32; d_y[b,k,h,w] = sum_c dout * (v1 - v0)
 // inside the clamp range (torch.clamp passes the gradient on the closed interval), accumulated across channel blocks.
+// Deterministic backward (mmu_snake_sample_bwd_det): gather-side, no float atomics - see snake_bwd_det_dfeat_kernel.
 #include "common.cuh"
 
 namespace mmu {
@@ -182,6 +183,139 @@ __global__ void __launch_bounds__(256) snake_bwd_nhwc_kernel(const TI *__restric
         atomicAdd(dy + (((int64_t)b * g.K + k) * g.H + h) * g.W + w, acc);
 }
 
+// ---- deterministic backward -------------------------------------------------------------------------------------------------
+// d_feat: the scatter targets are data-dependent rows, so the work is organised by TARGET column instead.  One thread owns the column
+// dfeat[b, c (or 4 channels), :, x] - nobody else writes it - and walks every sample that reads column x, i.e. every (k, h, w) with
+// clamp(w + k - K/2, 0, W-1) == x, in the fixed order k, h, w.  The two taps of consecutive samples mostly hit the same or the next
+// row, so they are summed in registers over a window of rows (rc, rc + 1) and added to global memory (plain read-modify-write) when
+// the window moves.  Consecutive threads own consecutive x (NCHW) or channel vectors (NHWC): the dout / y / dfeat accesses coalesce.
+// d_y: one thread per sample sums over ALL channels in channel order (snake_bwd_det_dy_kernel).
+__device__ __forceinline__ void snake_rowf(float yv, int H, int &r0, bool &r1ok, float &f, bool &inside) {
+    const float hi = (float)(H - 1);
+    const bool is_nan = yv != yv;                // as snake_coord: NaN poisons the sample and its gradients
+    inside = (yv >= 0.f && yv <= hi) || is_nan;
+    const float yc = fminf(fmaxf(yv, 0.f), hi);
+    const float fl = floorf(yc);
+    r0 = (int)fl;
+    f = is_nan ? yv : yc - fl;
+    r1ok = r0 + 1 < H;
+}
+
+template <int NV> struct RowWin {      // pending contributions to rows rc and rc + 1 of one owned column (NV channels)
+    int rc = -2;
+    float a0[NV] = {}, a1[NV] = {};
+    __device__ __forceinline__ void flush(float *col, int64_t rstride, int H) {
+        if (rc < 0) return;
+        float *p = col + (int64_t)rc * rstride;
+#pragma unroll
+        for (int i = 0; i < NV; ++i) p[i] += a0[i];
+        if (rc + 1 < H) {
+#pragma unroll
+            for (int i = 0; i < NV; ++i) p[rstride + i] += a1[i];
+        }
+    }
+    __device__ __forceinline__ void add(int r0, bool r1ok, float f, const float (&gv)[NV], float *col, int64_t rstride, int H) {
+        const float f0 = 1.f - f;
+        if (r0 == rc + 1) {              // the window slides by one row: row rc is complete
+            flush_row0(col, rstride);
+#pragma unroll
+            for (int i = 0; i < NV; ++i) a0[i] = a1[i], a1[i] = 0.f;
+            rc = r0;
+        } else if (r0 != rc) {
+            flush(col, rstride, H);
+#pragma unroll
+            for (int i = 0; i < NV; ++i) a0[i] = 0.f, a1[i] = 0.f;
+            rc = r0;
+        }
+#pragma unroll
+        for (int i = 0; i < NV; ++i) {
+            a0[i] = fmaf(f0, gv[i], a0[i]);
+            if (r1ok) a1[i] = fmaf(f, gv[i], a1[i]);
+        }
+    }
+    __device__ __forceinline__ void flush_row0(float *col, int64_t rstride) {
+        if (rc < 0) return;
+        float *p = col + (int64_t)rc * rstride;
+#pragma unroll
+        for (int i = 0; i < NV; ++i) p[i] += a0[i];
+    }
+};
+
+// NCHW: grid (x blocks, b*C + c); NHWC (NV = 4): grid (blocks over (x, channel vector), b)
+template <typename TO, bool NHWC>
+__global__ void __launch_bounds__(256) snake_bwd_det_dfeat_kernel(const float *__restrict__ y, const TO *__restrict__ dout,
+                                                                  float *__restrict__ dfeat, SnakeGeom g) {
+    constexpr int NV = NHWC ? 4 : 1;
+    const unsigned t = blockIdx.x * blockDim.x + threadIdx.x;
+    const int x = NHWC ? (int)(t >> g.cpb) : (int)t;
+    const int b = NHWC ? (int)blockIdx.y : (int)(blockIdx.y / (unsigned)g.C);
+    const int c = NHWC ? (int)(t & (((unsigned)g.C >> 2) - 1)) << 2 : (int)blockIdx.y - b * g.C;
+    if (x >= g.W) return;
+    const int H = g.H, W = g.W, K = g.K;
+    float *col = NHWC ? dfeat + ((int64_t)b * H * W + x) * g.C + c : dfeat + ((int64_t)b * g.C + c) * H * W + x;
+    const int64_t rstride = NHWC ? (int64_t)W * g.C : W;
+    RowWin<NV> win;
+    for (int k = 0; k < K; ++k) {
+        const int s = k - K / 2;
+        const int wa = x == 0 ? 0 : max(0, x - s), wb = x == W - 1 ? W - 1 : min(W - 1, x - s);
+        if (wa > wb) continue;
+        const float *yk = y + ((int64_t)b * K + k) * H * W;
+#pragma unroll 1
+        for (int h = 0; h < H; ++h) {
+#pragma unroll 1
+            for (int w = wa; w <= wb; ++w) {
+                int r0;
+                bool r1ok, inside;
+                float f, gv[NV];
+                snake_rowf(yk[(int64_t)h * W + w], H, r0, r1ok, f, inside);
+                if constexpr (NHWC) {
+                    Vec4<TO>::ld(dout + ((((int64_t)b * H + h) * K + k) * W + w) * g.C + c, gv);
+                } else {
+                    gv[0] = ldf(dout + (((int64_t)b * g.C + c) * H + h) * K * W + (int64_t)k * W + w);
+                }
+                win.add(r0, r1ok, f, gv, col, rstride, H);
+            }
+        }
+    }
+    win.flush(col, rstride, H);
+}
+
+// d_y[b,k,h,w] += sum over every channel, in channel order, of dout * (v1 - v0) (inside the clamp range).  Grid as snake_fwd_kernel
+// with one channel block (NCHW), or (output row, w blocks of 256) (NHWC).
+template <typename TI, typename TO, bool NHWC>
+__global__ void __launch_bounds__(256) snake_bwd_det_dy_kernel(const TI *__restrict__ feat, const float *__restrict__ y, const TO *__restrict__ dout,
+                                                               float *__restrict__ dy, SnakeGeom g) {
+    int b, h, k, r0, r1ok, xk;
+    float f;
+    bool inside;
+    const int w = blockIdx.y * blockDim.x + threadIdx.x;
+    if (w >= g.W) return;
+    snake_coord(g, y, blockIdx.x, w, b, h, k, r0, r1ok, f, xk, inside);
+    const int64_t plane = (int64_t)g.H * g.W;
+    float acc = 0.f;
+    if constexpr (NHWC) {
+        const TI *p0 = feat + (((int64_t)b * g.H + r0) * g.W + xk) * g.C;
+        const TO *go = dout + ((((int64_t)b * g.H + h) * g.K + k) * g.W + w) * g.C;
+        for (int c = 0; c < g.C; c += 4) {
+            float gv[4], v0[4], v1[4] = {0.f, 0.f, 0.f, 0.f};
+            Vec4<TO>::ld(go + c, gv);
+            Vec4<TI>::ld(p0 + c, v0);
+            if (r1ok) Vec4<TI>::ld(p0 + (int64_t)g.W * g.C + c, v1);
+#pragma unroll
+            for (int i = 0; i < 4; ++i) acc = fmaf(gv[i], v1[i] - v0[i], acc);
+        }
+    } else {
+        const TI *p0 = feat + (int64_t)b * g.C * plane + (int64_t)r0 * g.W + xk;
+        const TO *go = dout + (((int64_t)b * g.C) * g.H + h) * g.K * g.W + (int64_t)k * g.W + w;
+#pragma unroll 4
+        for (int c = 0; c < g.C; ++c, p0 += plane, go += plane * g.K) {
+            const float gv = ldf(go), v0 = ldf(p0);
+            acc = r1ok ? fmaf(gv, ldf(p0 + g.W) - v0, acc) : fmaf(gv, -v0, acc);
+        }
+    }
+    if (inside) dy[(((int64_t)b * g.K + k) * g.H + h) * g.W + w] += fmaf(f, 0.f, acc);   // NaN f -> NaN dy; one owner per sample
+}
+
 namespace {
 int geom_nhwc(SnakeGeom &g, int B, int C, int H, int W, int K, dim3 &grid, int &threads) {
     threads = 256;
@@ -288,4 +422,57 @@ extern "C" int mmu_snake_sample_bwd(const void *feat, const float *y, const void
         return set_error(MMU_ERR_UNSUPPORTED, "snake_sample_bwd: dtypes %d -> %d", in_dtype, out_dtype);
     count_launch();
     return check_launch("snake_sample_bwd");
+}
+
+// Deterministic backward: no workspace (every output element has exactly one writer); the query exists for a uniform interface.
+extern "C" size_t mmu_snake_sample_bwd_det_workspace(int32_t B, int32_t C, int32_t H, int32_t W, int32_t K, int32_t channels_last) {
+    (void)B, (void)C, (void)H, (void)W, (void)K, (void)channels_last;
+    return 0;
+}
+
+extern "C" int mmu_snake_sample_bwd_det(const void *feat, const float *y, const void *dout, float *dfeat, float *dy, int32_t in_dtype,
+                                        int32_t out_dtype, int32_t B, int32_t C, int32_t H, int32_t W, int32_t K, int32_t channels_last,
+                                        void *ws, size_t ws_bytes, void *stream) {
+    using namespace mmu;
+    (void)ws, (void)ws_bytes;
+    SnakeGeom g;
+    dim3 grid;
+    int nthr = 0;
+    if (int rc = channels_last ? geom_nhwc(g, B, C, H, W, K, grid, nthr) : geom(g, B, C, H, W, K, grid, nthr)) return rc;
+    if (!feat || !y || !dout || !dfeat) return set_error(MMU_ERR_INVALID, "snake_sample_bwd_det: null pointer");
+    const bool f32in = in_dtype == MMU_F32, f32out = out_dtype == MMU_F32;
+    if ((in_dtype != MMU_F32 && in_dtype != MMU_BF16) || (out_dtype != MMU_F32 && out_dtype != MMU_BF16))
+        return set_error(MMU_ERR_UNSUPPORTED, "snake_sample_bwd: dtypes %d -> %d", in_dtype, out_dtype);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const unsigned rows = (unsigned)((int64_t)B * H * K);
+    // d_feat by target column
+    if (channels_last) {
+        const int64_t per_b = (int64_t)W * (C / 4);
+        if ((per_b + 255) / 256 > 0x7fffffffLL || B > 65535) return set_error(MMU_ERR_UNSUPPORTED, "snake_sample_bwd_det: problem too large");
+        const dim3 dg((unsigned)((per_b + 255) / 256), (unsigned)B);
+        if (f32out) snake_bwd_det_dfeat_kernel<float, true><<<dg, 256, 0, st>>>(y, (const float *)dout, dfeat, g);
+        else snake_bwd_det_dfeat_kernel<__nv_bfloat16, true><<<dg, 256, 0, st>>>(y, (const __nv_bfloat16 *)dout, dfeat, g);
+    } else {
+        if ((int64_t)B * C > 65535) return set_error(MMU_ERR_UNSUPPORTED, "snake_sample_bwd_det: B * C > 65535");
+        const int nt = W >= 128 ? 128 : ((W + 31) / 32) * 32;
+        const dim3 dg((unsigned)((W + nt - 1) / nt), (unsigned)(B * C));
+        if (f32out) snake_bwd_det_dfeat_kernel<float, false><<<dg, nt, 0, st>>>(y, (const float *)dout, dfeat, g);
+        else snake_bwd_det_dfeat_kernel<__nv_bfloat16, false><<<dg, nt, 0, st>>>(y, (const __nv_bfloat16 *)dout, dfeat, g);
+    }
+    count_launch();
+    if (int rc = check_launch("snake_sample_bwd_det (d_feat)")) return rc;
+    if (dy == nullptr) return MMU_OK;
+    // d_y by sample, all channels in one thread
+    const int nt = channels_last ? 256 : nthr;
+    const dim3 yg(rows, (unsigned)((W + nt - 1) / nt));
+#define MMU_SNAKE_DY(TI_, TO_)                                                                                                         \
+    (channels_last ? snake_bwd_det_dy_kernel<TI_, TO_, true><<<yg, nt, 0, st>>>((const TI_ *)feat, y, (const TO_ *)dout, dy, g)         \
+                   : snake_bwd_det_dy_kernel<TI_, TO_, false><<<yg, nt, 0, st>>>((const TI_ *)feat, y, (const TO_ *)dout, dy, g))
+    if (f32in && f32out) MMU_SNAKE_DY(float, float);
+    else if (f32in) MMU_SNAKE_DY(float, __nv_bfloat16);
+    else if (f32out) MMU_SNAKE_DY(__nv_bfloat16, float);
+    else MMU_SNAKE_DY(__nv_bfloat16, __nv_bfloat16);
+#undef MMU_SNAKE_DY
+    count_launch();
+    return check_launch("snake_sample_bwd_det (d_y)");
 }

@@ -80,6 +80,14 @@ EXPORTS = (
     "mmu_group_norm_nhwc_fwd", "mmu_group_norm_nhwc_bwd",
     "mmu_mamba_narrow_supported", "mmu_mamba_narrow_rows", "mmu_mamba_narrow_weight_floats",
     "mmu_mamba_narrow_pre_fwd", "mmu_mamba_narrow_post_fwd", "mmu_mamba_narrow_post_bwd", "mmu_mamba_narrow_pre_bwd",
+    "mmu_deterministic_default",
+    "mmu_selective_scan_bwd_det_workspace", "mmu_selective_scan_bwd_det",
+    "mmu_causal_conv1d_bwd_det_workspace", "mmu_causal_conv1d_bwd_det",
+    "mmu_mamba_narrow_post_bwd_det_workspace", "mmu_mamba_narrow_pre_bwd_det_workspace",
+    "mmu_mamba_narrow_post_bwd_det", "mmu_mamba_narrow_pre_bwd_det",
+    "mmu_group_norm_nhwc_fwd_det_workspace", "mmu_group_norm_nhwc_bwd_det_workspace",
+    "mmu_group_norm_nhwc_fwd_det", "mmu_group_norm_nhwc_bwd_det",
+    "mmu_snake_sample_bwd_det_workspace", "mmu_snake_sample_bwd_det",
 )
 
 _lib = None
@@ -124,6 +132,23 @@ def lib() -> C.CDLL:
     L.mmu_mamba_narrow_weight_floats.argtypes = [_i32] * 5
     for n in ("mmu_mamba_narrow_pre_fwd", "mmu_mamba_narrow_post_fwd", "mmu_mamba_narrow_post_bwd", "mmu_mamba_narrow_pre_bwd"):
         getattr(L, n).argtypes = [C.POINTER(NarrowParams), _vp]
+    # deterministic mode: the plain entry point's arguments + (workspace, workspace bytes) before the stream
+    L.mmu_deterministic_default.restype = _i32
+    L.mmu_deterministic_default.argtypes = []
+    for n, args in (("mmu_selective_scan_bwd_det_workspace", [_i32] * 4), ("mmu_causal_conv1d_bwd_det_workspace", [_i32] * 4),
+                    ("mmu_mamba_narrow_post_bwd_det_workspace", [_i32] * 2), ("mmu_mamba_narrow_pre_bwd_det_workspace", [_i32] * 2),
+                    ("mmu_group_norm_nhwc_fwd_det_workspace", [_i32] * 4), ("mmu_group_norm_nhwc_bwd_det_workspace", [_i32] * 4)):
+        getattr(L, n).restype = _sz
+        getattr(L, n).argtypes = args
+    L.mmu_selective_scan_bwd_det.argtypes = [C.POINTER(ScanBwdParams), _vp, _sz, _vp]
+    L.mmu_causal_conv1d_bwd_det.argtypes = [C.POINTER(ConvParams), _vp, _sz, _vp]
+    for n in ("mmu_mamba_narrow_post_bwd_det", "mmu_mamba_narrow_pre_bwd_det"):
+        getattr(L, n).argtypes = [C.POINTER(NarrowParams), _vp, _sz, _vp]
+    L.mmu_group_norm_nhwc_fwd_det.argtypes = [_vp] * 7 + [_i32] * 6 + [C.c_float, _vp, _sz, _vp]
+    L.mmu_group_norm_nhwc_bwd_det.argtypes = [_vp] * 8 + [_i32] * 6 + [_vp, _sz, _vp]
+    L.mmu_snake_sample_bwd_det_workspace.restype = _sz
+    L.mmu_snake_sample_bwd_det_workspace.argtypes = [_i32] * 6
+    L.mmu_snake_sample_bwd_det.argtypes = [_vp, _vp, _vp, _vp, _vp] + [_i32] * 8 + [_vp, _sz, _vp]
     for n in EXPORTS:      # fail loudly on a stale library
         getattr(L, n)
     _lib = L

@@ -36,6 +36,24 @@ def _require_cuda(*ts):
             raise RuntimeError("mmunet_b200: expected CUDA tensors (there is no CPU path)")
 
 
+# Deterministic mode (include/mmunet_b200.h, "Deterministic mode"): every op below that sums floats across CTAs then calls its _det
+# entry point, which needs a workspace of partial-sum slots and gives bitwise reproducible results.
+_DET_SCAN_WS_CAP = 512 << 20      # bytes of scan-backward slots per call; larger problems run over batch slices
+
+
+def _deterministic() -> bool:
+    """True when torch.use_deterministic_algorithms(True) is on or the environment knob MMU_DETERMINISTIC is set (for callers that
+    cannot set torch's flag).  Checked when each kernel runs: backward functions at backward time."""
+    return torch.are_deterministic_algorithms_enabled() or bool(_lib.lib().mmu_deterministic_default())
+
+
+def _det_workspace(nbytes, device):
+    """-> (tensor, pointer, bytes): a fresh workspace for a _det entry point from the caching allocator of the current stream (its
+    contents do not matter: the kernels overwrite every slot they read)."""
+    ws = torch.empty(max(int(nbytes), 1), device=device, dtype=torch.uint8)
+    return ws, ws.data_ptr(), int(nbytes)
+
+
 # ----------------------------------------------------------------------------------------------------------
 # raw kernels
 # ----------------------------------------------------------------------------------------------------------
@@ -322,8 +340,33 @@ def _selective_scan_bwd_single(u, delta, A, B, C, D, z, delta_bias, dout, x, del
     dD = acc[2 * nBC + nA:2 * nBC + nA + dim] if D is not None else None
     dbias = acc[2 * nBC + nA + dim:] if delta_bias is not None else None
     L_ = _lib.lib()
+    det = _deterministic()
+    # deterministic mode: batch slices whose partial slots fit _DET_SCAN_WS_CAP (a function of the shape, so still reproducible);
+    # dA / dD / ddelta_bias then sum over the slices in slice order
+    nb = batch
+    if det:
+        while nb > 1 and L_.mmu_selective_scan_bwd_det_workspace(nb, H, L, N) > _DET_SCAN_WS_CAP:
+            nb = (nb + 1) // 2
+    for b0 in range(0, batch, nb):
+        sl = slice(b0, min(batch, b0 + nb))
+        _scan_bwd_launch(u[sl], delta[sl], A, B[sl], C[sl], D, z if z is None else z[sl], delta_bias, dout[sl], x[sl],
+                         None if y is None else y[sl], delta_softplus, reverse, du[sl], ddelta[sl], dz if dz is None else dz[sl],
+                         dB[sl], dC[sl], dA, dD, dbias, order, det)
+    return du, ddelta, dA, dB, dC, dD, dz, dbias
+
+
+def _scan_bwd_launch(u, delta, A, B, C, D, z, delta_bias, dout, x, y, delta_softplus, reverse, du, ddelta, dz, dB, dC, dA, dD, dbias,
+                     order, det):
+    """One mmu_selective_scan_bwd(_det) call per B/C group on prepared tensors (dB / dC: (batch, G, N, L) views)."""
+    batch, dim, L = u.shape
+    N = A.shape[1]
+    G = B.shape[1]
+    H = dim // G
+    L_ = _lib.lib()
     ws_bytes = L_.mmu_selective_scan_bwd_workspace(batch, H, L, N)
     ws = torch.empty(ws_bytes, device=u.device, dtype=torch.uint8) if ws_bytes else None
+    if det:
+        dws, dws_ptr, dws_bytes = _det_workspace(L_.mmu_selective_scan_bwd_det_workspace(batch, H, L, N), u.device)
     es = u.element_size()
     with torch.cuda.device(u.device):
         for g in range(G):
@@ -356,11 +399,13 @@ def _selective_scan_bwd_single(u, delta, A, B, C, D, z, delta_bias, dout, x, del
                 p.dB, p.dC = dBg.data_ptr(), dCg.data_ptr()
             p.dD = None if dD is None else dD.data_ptr() + g * H * 4
             p.ddelta_bias = None if dbias is None else dbias.data_ptr() + g * H * 4
-            _lib.check(L_.mmu_selective_scan_bwd(ct.byref(p), _stream()), "selective_scan_bwd")
+            if det:
+                _lib.check(L_.mmu_selective_scan_bwd_det(ct.byref(p), dws_ptr, dws_bytes, _stream()), "selective_scan_bwd_det")
+            else:
+                _lib.check(L_.mmu_selective_scan_bwd(ct.byref(p), _stream()), "selective_scan_bwd")
             if G > 1:
                 dB[:, g:g + 1] = dBg
                 dC[:, g:g + 1] = dCg
-    return du, ddelta, dA, dB, dC, dD, dz, dbias
 
 
 def _conv_params(x, weight, bias, silu, reverse=False, order=None):
@@ -419,8 +464,13 @@ def causal_conv1d_bwd(x, weight, bias, dout, silu=False, dx=None, reverse=False,
     p.dout, p.dout_bs, p.dout_ds = dout.data_ptr(), dout.stride(0), dout.stride(1)
     p.dx, p.dx_bs, p.dx_ds = dx.data_ptr(), dx.stride(0), dx.stride(1)
     p.dweight, p.dbias = dw.data_ptr(), _ptr(db)
+    L_ = _lib.lib()
     with torch.cuda.device(x.device):
-        _lib.check(_lib.lib().mmu_causal_conv1d_bwd(ct.byref(p), _stream()), "causal_conv1d_bwd")
+        if _deterministic():
+            ws, wp, wb = _det_workspace(L_.mmu_causal_conv1d_bwd_det_workspace(p.batch, p.dim, p.seqlen, p.dtype), x.device)
+            _lib.check(L_.mmu_causal_conv1d_bwd_det(ct.byref(p), wp, wb, _stream()), "causal_conv1d_bwd_det")
+        else:
+            _lib.check(L_.mmu_causal_conv1d_bwd(ct.byref(p), _stream()), "causal_conv1d_bwd")
     return dx, dw, db
 
 
@@ -959,6 +1009,10 @@ class MambaNarrowFn(torch.autograd.Function):
         dout_y = torch.empty((batch, di, L), device=hidden.device, dtype=io)
         gpre = torch.empty((batch, 3 * di, L), device=hidden.device, dtype=io)
         dhidden = torch.empty_like(hidden)
+        det = _deterministic()
+        if det:
+            dws, dws_ptr, dws_bytes = _det_workspace(max(L_.mmu_mamba_narrow_post_bwd_det_workspace(batch, L),
+                                                             L_.mmu_mamba_narrow_pre_bwd_det_workspace(batch, L)), hidden.device)
         with torch.cuda.device(hidden.device):
             p = _narrow_params(io, hidden.dtype, batch, L, ctx.dims, ctx.order, ws, coord)
             p.out_z, p.dout_y, p.dweights = out_z.data_ptr(), dout_y.data_ptr(), dW.data_ptr()
@@ -966,7 +1020,10 @@ class MambaNarrowFn(torch.autograd.Function):
                 p.dcoords = dout.data_ptr()
             else:
                 p.dout, p.dout_bs, p.dout_cs = dout.data_ptr(), dout.stride(0), dout.stride(1)
-            _lib.check(L_.mmu_mamba_narrow_post_bwd(ct.byref(p), _stream()), "mamba_narrow_post_bwd")
+            if det:
+                _lib.check(L_.mmu_mamba_narrow_post_bwd_det(ct.byref(p), dws_ptr, dws_bytes, _stream()), "mamba_narrow_post_bwd_det")
+            else:
+                _lib.check(L_.mmu_mamba_narrow_post_bwd(ct.byref(p), _stream()), "mamba_narrow_post_bwd")
             u, delta, z = pre[:, :di], pre[:, di:2 * di], pre[:, 2 * di:3 * di]
             Bm, Cm = pre[:, 3 * di:3 * di + N].unsqueeze(1), pre[:, 3 * di + N:].unsqueeze(1)
             _, _, dA, _, _, dD, _, ddt_bias = selective_scan_bwd(
@@ -975,7 +1032,10 @@ class MambaNarrowFn(torch.autograd.Function):
             p.hidden, p.hidden_bs, p.hidden_cs, p.pre = hidden.data_ptr(), hidden.stride(0), hidden.stride(1), pre.data_ptr()
             p.gpre, p.dBC = gpre.data_ptr(), dBC.data_ptr()
             p.dhidden, p.dhidden_bs, p.dhidden_cs = dhidden.data_ptr(), dhidden.stride(0), dhidden.stride(1)
-            _lib.check(L_.mmu_mamba_narrow_pre_bwd(ct.byref(p), _stream()), "mamba_narrow_pre_bwd")
+            if det:
+                _lib.check(L_.mmu_mamba_narrow_pre_bwd_det(ct.byref(p), dws_ptr, dws_bytes, _stream()), "mamba_narrow_pre_bwd_det")
+            else:
+                _lib.check(L_.mmu_mamba_narrow_pre_bwd(ct.byref(p), _stream()), "mamba_narrow_pre_bwd")
         sizes = (2 * di * dm, di * kw, di, (R + 2 * N) * di, di * R, dm * di, 1)
         g_in, g_cw, g_cb, g_x, g_dt, g_out, g_al = torch.split(dW, sizes)
         wd = ctx.wdtypes
@@ -1104,10 +1164,15 @@ class _SnakeSampleFn(torch.autograd.Function):
         acc = torch.zeros(nf + y.numel(), device=feat.device, dtype=torch.float32)     # one zero fill for both accumulators
         dfeat = acc[:nf].view(B, H, W, C_).permute(0, 3, 1, 2) if ctx.cl else acc[:nf].view(B, C_, H, W)
         dy = acc[nf:].view_as(y)
+        L_ = _lib.lib()
+        args = (feat.data_ptr(), y.data_ptr(), dout.data_ptr(), dfeat.data_ptr(), dy.data_ptr(), _DT[feat.dtype], _DT[ctx.out_dtype],
+                B, C_, H, W, K, int(ctx.cl))
         with torch.cuda.device(feat.device):
-            _lib.check(_lib.lib().mmu_snake_sample_bwd(feat.data_ptr(), y.data_ptr(), dout.data_ptr(), dfeat.data_ptr(), dy.data_ptr(),
-                                                       _DT[feat.dtype], _DT[ctx.out_dtype], B, C_, H, W, K, int(ctx.cl), _stream()),
-                       "snake_sample_bwd")
+            if _deterministic():
+                ws, wp, wb = _det_workspace(L_.mmu_snake_sample_bwd_det_workspace(B, C_, H, W, K, int(ctx.cl)), feat.device)
+                _lib.check(L_.mmu_snake_sample_bwd_det(*args, wp, wb, _stream()), "snake_sample_bwd_det")
+            else:
+                _lib.check(L_.mmu_snake_sample_bwd(*args, _stream()), "snake_sample_bwd")
         return dfeat.to(feat.dtype), dy, None
 
 
@@ -1137,10 +1202,15 @@ class _GroupNormNhwcFn(torch.autograd.Function):
         y = torch.empty((B, C_, H, W), device=x.device, dtype=out_dtype, memory_format=torch.channels_last)
         stats = torch.zeros(4 * B * G, device=x.device, dtype=torch.float32)          # sums (2BG) | mean (BG) | rstd (BG)
         sums, mean, rstd = stats[:2 * B * G], stats[2 * B * G:3 * B * G], stats[3 * B * G:]
+        L_ = _lib.lib()
+        args = (x.data_ptr(), w32.data_ptr(), b32.data_ptr(), y.data_ptr(), sums.data_ptr(), mean.data_ptr(), rstd.data_ptr(), _DT[x.dtype],
+                _DT[out_dtype], B, C_, H * W, G, float(eps))
         with torch.cuda.device(x.device):
-            _lib.check(_lib.lib().mmu_group_norm_nhwc_fwd(x.data_ptr(), w32.data_ptr(), b32.data_ptr(), y.data_ptr(), sums.data_ptr(),
-                                                          mean.data_ptr(), rstd.data_ptr(), _DT[x.dtype], _DT[out_dtype], B, C_, H * W, G,
-                                                          float(eps), _stream()), "group_norm_nhwc_fwd")
+            if _deterministic():
+                ws, wp, wb = _det_workspace(L_.mmu_group_norm_nhwc_fwd_det_workspace(B, C_, H * W, G), x.device)
+                _lib.check(L_.mmu_group_norm_nhwc_fwd_det(*args, wp, wb, _stream()), "group_norm_nhwc_fwd_det")
+            else:
+                _lib.check(L_.mmu_group_norm_nhwc_fwd(*args, _stream()), "group_norm_nhwc_fwd")
         ctx.save_for_backward(x, w32, mean, rstd)
         ctx.G, ctx.out_dtype, ctx.wdtype = G, out_dtype, weight.dtype
         return y
@@ -1153,10 +1223,15 @@ class _GroupNormNhwcFn(torch.autograd.Function):
         dy = dy.to(ctx.out_dtype).contiguous(memory_format=torch.channels_last)
         dx = torch.empty_like(x, memory_format=torch.channels_last)
         acc = torch.zeros(2 * B * G + 2 * C_, device=x.device, dtype=torch.float32)    # S1,S2 per (b, group) | dgamma | dbeta
+        L_ = _lib.lib()
+        args = (x.data_ptr(), w32.data_ptr(), dy.data_ptr(), mean.data_ptr(), rstd.data_ptr(), dx.data_ptr(), acc.data_ptr(),
+                acc[2 * B * G:].data_ptr(), _DT[x.dtype], _DT[ctx.out_dtype], B, C_, H * W, G)
         with torch.cuda.device(x.device):
-            _lib.check(_lib.lib().mmu_group_norm_nhwc_bwd(x.data_ptr(), w32.data_ptr(), dy.data_ptr(), mean.data_ptr(), rstd.data_ptr(),
-                                                          dx.data_ptr(), acc.data_ptr(), acc[2 * B * G:].data_ptr(), _DT[x.dtype],
-                                                          _DT[ctx.out_dtype], B, C_, H * W, G, _stream()), "group_norm_nhwc_bwd")
+            if _deterministic():
+                ws, wp, wb = _det_workspace(L_.mmu_group_norm_nhwc_bwd_det_workspace(B, C_, H * W, G), x.device)
+                _lib.check(L_.mmu_group_norm_nhwc_bwd_det(*args, wp, wb, _stream()), "group_norm_nhwc_bwd_det")
+            else:
+                _lib.check(L_.mmu_group_norm_nhwc_bwd(*args, _stream()), "group_norm_nhwc_bwd")
         dgamma, dbeta = acc[2 * B * G:2 * B * G + C_], acc[2 * B * G + C_:]
         return dx, dgamma.to(ctx.wdtype), dbeta.to(ctx.wdtype), None, None, None
 
