@@ -319,6 +319,15 @@ size_t mmu_snake_sample_bwd_det_workspace(int32_t B, int32_t C, int32_t H, int32
 int mmu_snake_sample_bwd_det(const void *feat, const float *y, const void *dout, float *dfeat, float *dy, int32_t in_dtype,
                              int32_t out_dtype, int32_t B, int32_t C, int32_t H, int32_t W, int32_t K, int32_t channels_last, void *ws,
                              size_t ws_bytes, void *stream);
+/* bilinear-resize backward: the adjoint of F.interpolate(x, size=(H_out, W_out), mode="bilinear", align_corners=True) for a
+ * (B, C, H_in, W_in) map, dx from dout (B, C, H_out, W_out).  dout and dx share the dtype (MMU_F32 or MMU_BF16) and the layout: dense
+ * NCHW, or NHWC when channels_last != 0.  Gather-side: every dx element is written exactly once (no zero-fill, no workspace) with the
+ * sum, in fp32 and in a fixed order (output row, then output column, ascending), of dout times the forward's weights, recomputed as
+ * ATen computes them (scale (in - 1) / (out - 1) in fp32, 0 when out == 1), and rounded once to the dtype.  MMU_ERR_INVALID, before
+ * anything is enqueued, for NULL pointers, another dtype, a size <= 0, or more elements than the kernels index (H_in * W_in and
+ * H_out * W_out, times ceil(C / 16-byte vector) for NHWC input pixels, must fit int32; B * C * H * W must fit int64). */
+int mmu_resize_bilinear_bwd_det(const void *dout, void *dx, int32_t dtype, int32_t B, int32_t C, int32_t H_in, int32_t W_in,
+                                int32_t H_out, int32_t W_out, int32_t channels_last, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
  * misc

@@ -88,6 +88,7 @@ EXPORTS = (
     "mmu_group_norm_nhwc_fwd_det_workspace", "mmu_group_norm_nhwc_bwd_det_workspace",
     "mmu_group_norm_nhwc_fwd_det", "mmu_group_norm_nhwc_bwd_det",
     "mmu_snake_sample_bwd_det_workspace", "mmu_snake_sample_bwd_det",
+    "mmu_resize_bilinear_bwd_det",
 )
 
 _lib = None
@@ -149,6 +150,7 @@ def lib() -> C.CDLL:
     L.mmu_snake_sample_bwd_det_workspace.restype = _sz
     L.mmu_snake_sample_bwd_det_workspace.argtypes = [_i32] * 6
     L.mmu_snake_sample_bwd_det.argtypes = [_vp, _vp, _vp, _vp, _vp] + [_i32] * 8 + [_vp, _sz, _vp]
+    L.mmu_resize_bilinear_bwd_det.argtypes = [_vp, _vp] + [_i32] * 8 + [_vp]
     for n in EXPORTS:      # fail loudly on a stale library
         getattr(L, n)
     _lib = L

@@ -22,6 +22,8 @@ What differs from the reference (performance only, same arithmetic):
     (SURVEY.md section 0.5) - tensors follow the input's device;
   * `Mamba` is `mmunet_b200.mamba.Mamba` (hosts bimamba_type="v1", which the reference constructor rejects,
     SURVEY.md section 0.4).
+  * the bilinear resizes (F.interpolate, align_corners=True) go through `ops.resize_bilinear`: the same call, except that in
+    deterministic mode their backward is the library's gather-side kernel instead of ATen's atomic scatter.
 `MM_Net` is the only model of the reference's zoo built here: it is the one that calls the hot path.
 """
 from __future__ import annotations
@@ -202,7 +204,7 @@ class RCG(nn.Module):
 
     def forward(self, pre, edge, f):
         r = (1.0 - torch.sigmoid(pre)) * f                                               # (:390-392)
-        edge1 = F.interpolate(edge, size=f.shape[2:], mode="bilinear", align_corners=True)
+        edge1 = ops.resize_bilinear(edge, size=f.shape[2:])
         x2 = self.conv1(torch.cat((edge1, r), 1))
         x0 = self.upsample(x2)
         B, C, H, W = x0.shape
@@ -221,7 +223,7 @@ class DecoderBlock(nn.Module):
         self.conv2 = _mm_bn_relu(in_channels // 4, out_channels, num_slices)
 
     def forward(self, x):
-        return F.interpolate(self.conv2(self.conv1(x)), scale_factor=2, mode="bilinear", align_corners=True)
+        return ops.resize_bilinear(self.conv2(self.conv1(x)), scale_factor=2)
 
 
 class ResidualBlock(nn.Module):
@@ -306,7 +308,7 @@ class MM_Net(nn.Module):
         out2 = self.side2(d2)
         total = None
         for t in (out2, out3, out4, out5, p_c):              # (:577)
-            up = F.interpolate(t, size=size, mode="bilinear", align_corners=True)
+            up = ops.resize_bilinear(t, size=size)
             total = up if total is None else total + up
         return total
 

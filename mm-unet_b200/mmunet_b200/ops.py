@@ -1242,3 +1242,48 @@ def group_norm_nhwc(x, num_groups, weight, bias, eps=1e-5, out_dtype=None):
     if not group_norm_nhwc_supported(x, num_groups):
         raise RuntimeError("group_norm_nhwc: needs a CUDA channels-last (B, 4*G, H, W) fp32/bf16 tensor with G | 256 or G >= 256")
     return _GroupNormNhwcFn.apply(x, weight, bias, num_groups, eps, x.dtype if out_dtype is None else out_dtype)
+
+
+# ----------------------------------------------------------------------------------------------------------
+# bilinear resize (align_corners=True): deterministic backward for MM_Net's three F.interpolate sites
+# ----------------------------------------------------------------------------------------------------------
+
+def resize_bilinear_bwd(dout, in_hw, channels_last):
+    """dout (B, C, Ho, Wo) fp32 / bf16 -> dx (B, C, *in_hw) in dout's dtype: the adjoint of F.interpolate(..., mode="bilinear",
+    align_corners=True), gather-side (mmu_resize_bilinear_bwd_det: no atomics, the same bits on every run).  channels_last picks the
+    NHWC kernel; dx then has channels-last strides."""
+    _require_cuda(dout)
+    if dout.dtype not in (torch.float32, torch.bfloat16) or dout.dim() != 4:
+        raise RuntimeError("resize_bilinear_bwd: needs a 4-D float32 or bfloat16 tensor")
+    fmt = torch.channels_last if channels_last else torch.contiguous_format
+    dout = dout.contiguous(memory_format=fmt)
+    B, C_, Ho, Wo = dout.shape
+    Hi, Wi = in_hw
+    dx = torch.empty((B, C_, Hi, Wi), device=dout.device, dtype=dout.dtype, memory_format=fmt)
+    with torch.cuda.device(dout.device):
+        _lib.check(_lib.lib().mmu_resize_bilinear_bwd_det(dout.data_ptr(), dx.data_ptr(), _DT[dout.dtype], B, C_, Hi, Wi, Ho, Wo,
+                                                          int(bool(channels_last)), _stream()), "resize_bilinear_bwd_det")
+    return dx
+
+
+class _ResizeBilinearFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, size, scale_factor):
+        ctx.in_hw = tuple(x.shape[2:])
+        ctx.cl = not x.is_contiguous()           # dense channels-last (resize_bilinear checked the layout)
+        return F.interpolate(x, size=size, scale_factor=scale_factor, mode="bilinear", align_corners=True)
+
+    @staticmethod
+    def backward(ctx, dout):
+        return resize_bilinear_bwd(dout, ctx.in_hw, ctx.cl), None, None
+
+
+def resize_bilinear(x, size=None, scale_factor=None):
+    """F.interpolate(x, size, scale_factor, mode="bilinear", align_corners=True).  In deterministic mode (see _deterministic), for a
+    CUDA fp32 / bf16 map that is dense NCHW or channels-last, the backward is this library's gather-side kernel (ATen's scatters with
+    atomics, and torch refuses it under use_deterministic_algorithms(True)); dx keeps x's memory format.  Otherwise this is exactly
+    the F.interpolate call."""
+    if (x.is_cuda and x.dim() == 4 and x.dtype in (torch.float32, torch.bfloat16)
+            and (x.is_contiguous() or x.is_contiguous(memory_format=torch.channels_last)) and _deterministic()):
+        return _ResizeBilinearFn.apply(x, size, scale_factor)
+    return F.interpolate(x, size=size, scale_factor=scale_factor, mode="bilinear", align_corners=True)

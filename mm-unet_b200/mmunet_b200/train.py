@@ -66,6 +66,20 @@ def make_optimizer(model, lr=1e-3, weight_decay=0.05, betas=(0.9, 0.95), captura
     return torch.optim.AdamW(groups, lr=lr, betas=betas, fused=fused, capturable=capturable)
 
 
+CUBLAS_DETERMINISTIC_CONFIGS = (":4096:8", ":16:8")
+
+
+def check_deterministic_cublas():
+    """Under torch.use_deterministic_algorithms(True) (strict, not warn_only) torch refuses cuBLAS calls unless CUBLAS_WORKSPACE_CONFIG
+    is one of CUBLAS_DETERMINISTIC_CONFIGS, and MM_Net's projections use cuBLAS.  Raise here, at construction, instead of in the first
+    step (or in the middle of a CUDA-graph capture).  The variable must be set before the process first uses cuBLAS."""
+    if (torch.are_deterministic_algorithms_enabled() and not torch.is_deterministic_algorithms_warn_only_enabled()
+            and os.environ.get("CUBLAS_WORKSPACE_CONFIG") not in CUBLAS_DETERMINISTIC_CONFIGS):
+        raise RuntimeError("Trainer: torch.use_deterministic_algorithms(True) needs CUBLAS_WORKSPACE_CONFIG=:4096:8 (or :16:8) in the "
+                           "environment before the process first uses cuBLAS; it is "
+                           f"{os.environ.get('CUBLAS_WORKSPACE_CONFIG')!r}")
+
+
 class Trainer:
     """One rank of a (possibly data-parallel) synthetic-data MM_Net training job.
 
@@ -82,6 +96,8 @@ class Trainer:
         self.image_size, self.batch = image_size, batch_per_rank
         self.channels_last = channels_last
         self.is_cuda = self.device.type == "cuda"       # "cpu" only works with the tests' oracle stand-ins for the Mamba ops
+        if self.is_cuda:
+            check_deterministic_cublas()
         self.stream = torch.cuda.Stream(self.device) if self.is_cuda else None    # all training work runs on this side stream
         torch.manual_seed(seed)                                           # same initial weights on every rank (train.py:160)
         net = MM_Net(num_classes=1).to(self.device)
