@@ -330,6 +330,53 @@ int mmu_resize_bilinear_bwd_det(const void *dout, void *dx, int32_t dtype, int32
                                 int32_t H_out, int32_t W_out, int32_t channels_last, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Sliding-window stitch of MM_Net's five head maps (out2, out3, out4, out5, p_c): the window blending of monai's
+ * SlidingWindowInferer(roi_size = roi, overlap, mode="constant") as used by the reference's validation (train.py:180), with the
+ * model's own final resize-and-sum (MMUNet.py:577) fused in.  Per axis of the zero-padded image (size n >= roi):
+ *   interval = roi if n == roi, else max((int)(roi * (1 - overlap)), 1)   (the caller passes it; 1 <= interval <= roi)
+ *   count    = 1 + the first d >= 0 with d * interval + roi >= n;   window d starts at min(d * interval, n - roi)
+ *   windows are numbered row-major (row window index first); the image sits at (pad_top, pad_left) of the padded one.
+ * For every pixel (y, x) of the un-padded H x W image, in padded coordinates (y + pad_top, x + pad_left), and for every window
+ * covering it, in window order, with (a, b) the window-local coordinate:
+ *   v = up(out2) + up(out3) + up(out4) + up(out5) + up(p_c)   (fp32, in that order)
+ *   up(m) = F.interpolate(m, (roi, roi), mode="bilinear", align_corners=True)[a, b] computed as ATen does (scale (h_m - 1) / (roi - 1)
+ *           in fp32, 0 when roi == 1);   acc += v
+ * and logits[b][y][x] = acc / (number of covering windows), fp32.  Every logit is written once, without float atomics: the same bits
+ * on every run, on any stream and in CUDA-graph replays.
+ *   heads[k]  : C = 1 maps of head_h[k] x head_w[k], dtype `dtype` (MMU_F32 or MMU_BF16), column stride 1; the map of window w of
+ *               image i at heads[k] + i * head_bs[k] + w * head_ws[k] (+ row * head_rs[k] + column), element strides >= 0.
+ *   logits    : (batch, H, W) fp32, strides (logits_bs, logits_rs, 1).
+ *   target, fov: uint8 (batch, H, W) maps with their own strides, or NULL; target is required with counts.
+ *   counts    : int64 [batch][4] or NULL, ACCUMULATED INTO (caller zero-fills): TP, FP, FN, TN over the pixels with fov != 0 (all
+ *               pixels without fov), positive meaning logit > 0 and target != 0.  Per-block sums added with 64-bit integer atomics.
+ * MMU_ERR_INVALID, before anything is enqueued, for a NULL required pointer, another dtype, a size <= 0, n < roi, a pad outside
+ * [0, n - size], an interval outside [1, roi], a negative stride, or offsets / grid sizes the kernel cannot index (batch and
+ * ceil(H / 8) <= 65535, element offsets within int64).
+ * --------------------------------------------------------------------------------------------- */
+#define MMU_SW_HEADS 5
+typedef struct mmu_sw_stitch_params {
+    int32_t dtype;                       /* of the head maps */
+    int32_t batch;                       /* images of the same size */
+    int32_t H, W;                        /* image size: logits, target, fov */
+    int32_t roi;                         /* window side */
+    int32_t n_h, n_w;                    /* padded image size (>= roi) */
+    int32_t pad_top, pad_left;           /* zeros before the image in the padded one */
+    int32_t interval_h, interval_w;      /* window stride per axis */
+    int32_t head_h[MMU_SW_HEADS], head_w[MMU_SW_HEADS];
+    const void *heads[MMU_SW_HEADS];
+    int64_t head_bs[MMU_SW_HEADS], head_ws[MMU_SW_HEADS], head_rs[MMU_SW_HEADS];
+    float *logits;
+    int64_t logits_bs, logits_rs;
+    const uint8_t *target;
+    int64_t target_bs, target_rs;
+    const uint8_t *fov;
+    int64_t fov_bs, fov_rs;
+    int64_t *counts;
+} mmu_sw_stitch_params;
+
+int mmu_sw_stitch(const mmu_sw_stitch_params *p, void *stream);
+
+/* ---------------------------------------------------------------------------------------------
  * misc
  * --------------------------------------------------------------------------------------------- */
 int mmu_version(void);

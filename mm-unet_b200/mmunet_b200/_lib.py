@@ -70,6 +70,22 @@ class NarrowParams(C.Structure):
     )
 
 
+SW_HEADS = 5
+
+
+class SwStitchParams(C.Structure):
+    """mmu_sw_stitch_params (include/mmunet_b200.h)."""
+    _fields_ = (
+        [(n, _i32) for n in ("dtype", "batch", "H", "W", "roi", "n_h", "n_w", "pad_top", "pad_left", "interval_h", "interval_w")]
+        + [("head_h", _i32 * SW_HEADS), ("head_w", _i32 * SW_HEADS), ("heads", _vp * SW_HEADS)]
+        + [(n, _i64 * SW_HEADS) for n in ("head_bs", "head_ws", "head_rs")]
+        + [("logits", _vp), ("logits_bs", _i64), ("logits_rs", _i64)]
+        + [("target", _vp), ("target_bs", _i64), ("target_rs", _i64)]
+        + [("fov", _vp), ("fov_bs", _i64), ("fov_rs", _i64)]
+        + [("counts", _vp)]
+    )
+
+
 EXPORTS = (
     "mmu_version", "mmu_last_error", "mmu_launch_count", "mmu_reload_knobs",
     "mmu_selective_scan_fwd_workspace", "mmu_selective_scan_fwd",
@@ -89,6 +105,7 @@ EXPORTS = (
     "mmu_group_norm_nhwc_fwd_det", "mmu_group_norm_nhwc_bwd_det",
     "mmu_snake_sample_bwd_det_workspace", "mmu_snake_sample_bwd_det",
     "mmu_resize_bilinear_bwd_det",
+    "mmu_sw_stitch",
 )
 
 _lib = None
@@ -151,6 +168,7 @@ def lib() -> C.CDLL:
     L.mmu_snake_sample_bwd_det_workspace.argtypes = [_i32] * 6
     L.mmu_snake_sample_bwd_det.argtypes = [_vp, _vp, _vp, _vp, _vp] + [_i32] * 8 + [_vp, _sz, _vp]
     L.mmu_resize_bilinear_bwd_det.argtypes = [_vp, _vp] + [_i32] * 8 + [_vp]
+    L.mmu_sw_stitch.argtypes = [C.POINTER(SwStitchParams), _vp]
     for n in EXPORTS:      # fail loudly on a stale library
         getattr(L, n)
     _lib = L

@@ -288,7 +288,15 @@ class MM_Net(nn.Module):
         self.decoder2 = DecoderBlock(in_channels=128, out_channels=64, num_slices=ns[0])
 
     def forward(self, x):
-        size = x.shape[2:]
+        total = None
+        for t in self.forward_heads(x):                      # (:577)
+            up = ops.resize_bilinear(t, size=x.shape[2:])
+            total = up if total is None else total + up
+        return total
+
+    def forward_heads(self, x):
+        """The five (B, 1, h, w) logit maps (out2, out3, out4, out5, p_c) of a (B, 3, H, W) input, at 1/2, 1/4, 1/8, 1/16 and 1/2 of
+        its size, before forward's bilinear resize to (H, W) and sum (what the sliding-window predictor stitches)."""
         e1 = self.encoder1(x)
         e2 = self.encoder2(self.maxpool(e1))
         e3 = self.encoder3(e2)
@@ -306,11 +314,7 @@ class MM_Net(nn.Module):
         out3 = self.side3(d3)
         d2 = self.decoder2(torch.cat((d3, self.rcg2(out3, c1, e2)), dim=1))
         out2 = self.side2(d2)
-        total = None
-        for t in (out2, out3, out4, out5, p_c):              # (:577)
-            up = ops.resize_bilinear(t, size=size)
-            total = up if total is None else total + up
-        return total
+        return out2, out3, out4, out5, p_c
 
     def unused_parameters(self):
         """Parameters that never receive a gradient in MM_Net: the `_b`/`_s` sets of the v1 Mambas and `dsc_conv_y`

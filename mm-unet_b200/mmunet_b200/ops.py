@@ -13,6 +13,7 @@ raises RuntimeError.
 from __future__ import annotations
 
 import ctypes as ct
+import threading
 
 import torch
 import torch.nn.functional as F
@@ -208,7 +209,9 @@ def _selective_scan_fwd_single(u, delta, A, B, C, D=None, z=None, delta_bias=Non
     out = torch.empty_like(u, memory_format=torch.contiguous_format)
     H = dim // G
     L_ = _lib.lib()
-    xs = L_.mmu_scan_state_stride(batch, H, L, N, _DT[u.dtype]) if (save_states and order is None) else _lib.STATE_STRIDE
+    # the state stride takes part in the kernel choice (fwd5 / fwd4 eligibility): it is the same with and without saved states, so a
+    # forward-only call runs the kernel the grad-saving call runs
+    xs = L_.mmu_scan_state_stride(batch, H, L, N, _DT[u.dtype]) if order is None else _lib.STATE_STRIDE
     nx = (L + xs - 1) // xs
     x = torch.empty((batch, dim, nx, N), device=u.device, dtype=torch.float32) if save_states else None
     y = torch.empty_like(out) if (save_states and z is not None) else None
@@ -499,7 +502,34 @@ def _load(ctx):
     return tuple(None if k is None else (next(it) if k == -1 else [next(it) for _ in range(k)]) for k in ctx.saved_spec)
 
 
-class SelectiveScanFn(torch.autograd.Function):
+_FWD_TLS = threading.local()
+
+
+def _saving() -> bool:
+    """Inside the forward of a _ForwardOnlyAware Function: False when its call records no autograd graph (grad mode off, or no tensor
+    argument requires grad), so nothing the backward needs has to be stored."""
+    return getattr(_FWD_TLS, "save", True)
+
+
+class _ForwardOnlyAware(torch.autograd.Function):
+    """Base of the Mamba Functions with a forward-only path.  torch runs forward() with grad mode off and ctx.needs_input_grad does not
+    see the caller's grad mode, so apply() records, for forward(), whether this call will ever be differentiated.  When it will not,
+    the scan runs with save_states=False - the same kernel without the stores of the state snapshots x and the pre-gate y - and
+    nothing is saved on ctx, so the forward's intermediates are freed when it returns.  The outputs are bitwise those of the
+    grad-saving call."""
+
+    @classmethod
+    def apply(cls, *args, **kwargs):
+        prev = getattr(_FWD_TLS, "save", True)
+        _FWD_TLS.save = torch.is_grad_enabled() and any(isinstance(a, torch.Tensor) and a.requires_grad
+                                                         for a in (*args, *kwargs.values()))
+        try:
+            return super().apply(*args, **kwargs)
+        finally:
+            _FWD_TLS.save = prev
+
+
+class SelectiveScanFn(_ForwardOnlyAware):
     """selective_scan_interface.py:14-74."""
 
     @staticmethod
@@ -523,11 +553,13 @@ class SelectiveScanFn(torch.autograd.Function):
             B = B.unsqueeze(1)
         if ctx.squeeze_C:
             C = C.unsqueeze(1)
+        save = _saving()
         out, x, last = selective_scan_fwd(u, delta, A, B, C, D, z, delta_bias, delta_softplus,
-                                          save_states=True, return_last_state=return_last_state)
+                                          save_states=save, return_last_state=return_last_state)
         ctx.delta_softplus = delta_softplus
         ctx.has_z = z is not None
-        _save(ctx, (u, delta, A, B, C, D, z, delta_bias, x.x, x.y))
+        if save:
+            _save(ctx, (u, delta, A, B, C, D, z, delta_bias, x.x, x.y))
         return out if not return_last_state else (out, last)
 
     @staticmethod
@@ -596,7 +628,7 @@ class _InnerCore:
 
     @staticmethod
     def forward(xz, conv1d_weight, conv1d_bias, x_proj_weight, delta_proj_weight, A, B, C, D, delta_bias,
-                B_proj_bias, C_proj_bias, delta_softplus, reverse=False, order=None):
+                B_proj_bias, C_proj_bias, delta_softplus, reverse=False, order=None, save_states=True):
         """order = (kind, H, W, nslices): the scan runs over xz in that token order WITHOUT permuted copies - the conv reads x
         through the index map and writes conv_out in scan order, the projections work on scan-order tensors (they are per-token),
         the scan reads the gate z and writes its output through the map: out_z comes back in natural token order
@@ -623,9 +655,10 @@ class _InnerCore:
         Bm = x3[R:R + N].permute(1, 0, 2).unsqueeze(1)                              # (b, 1, n, l) views of x_dbl
         Cm = x3[R + N:].permute(1, 0, 2).unsqueeze(1)
         D = D.contiguous() if D is not None else None
-        out_z, xs, _ = selective_scan_fwd(conv_out, delta, A, Bm, Cm, D, z, delta_bias, delta_softplus, reverse=reverse, order=order)
+        out_z, xs, _ = selective_scan_fwd(conv_out, delta, A, Bm, Cm, D, z, delta_bias, delta_softplus, reverse=reverse, order=order,
+                                          save_states=save_states)
         saved = (xz, conv_w, conv_b, x_dbl, x_proj_weight, delta_proj_weight, conv_st, delta, A, None, None, D, delta_bias,
-                 xs.x, xs.y)
+                 xs.x if save_states else None, xs.y if save_states else None)
         return out_z, saved
 
     @staticmethod
@@ -729,7 +762,7 @@ def _cast_proj(*ws):
     return tuple(w.to(dt) if (dt is not None and w is not None) else w for w in ws)
 
 
-class MambaInnerFnNoOutProj(torch.autograd.Function):
+class MambaInnerFnNoOutProj(_ForwardOnlyAware):
     """selective_scan_interface.py:155-289 (returns out_z (b, d, l))."""
 
     @staticmethod
@@ -738,12 +771,15 @@ class MambaInnerFnNoOutProj(torch.autograd.Function):
                 delta_bias=None, B_proj_bias=None, C_proj_bias=None, delta_softplus=True, checkpoint_lvl=1,
                 reverse=False, order=None):
         x_proj_weight, delta_proj_weight = _cast_proj(x_proj_weight, delta_proj_weight)
+        save = _saving()
         out_z, saved = _InnerCore.forward(xz, conv1d_weight, conv1d_bias, x_proj_weight, delta_proj_weight, A, B, C, D,
-                                          delta_bias, B_proj_bias, C_proj_bias, delta_softplus, reverse=reverse, order=order)
+                                          delta_bias, B_proj_bias, C_proj_bias, delta_softplus, reverse=reverse, order=order,
+                                          save_states=save)
         ctx.delta_softplus = delta_softplus
         ctx.reverse = reverse
         ctx.order = order
-        _save(ctx, saved)
+        if save:
+            _save(ctx, saved)
         return out_z
 
     @staticmethod
@@ -754,7 +790,7 @@ class MambaInnerFnNoOutProj(torch.autograd.Function):
         return (dxz, dcw, dcb, dxw, ddw, dA, None, None, dD, ddb, None, None, None, None, None, None)
 
 
-class MambaInnerFn(torch.autograd.Function):
+class MambaInnerFn(_ForwardOnlyAware):
     """selective_scan_interface.py:292-434 (fused out_proj; returns (b, l, d_model))."""
 
     @staticmethod
@@ -764,13 +800,14 @@ class MambaInnerFn(torch.autograd.Function):
                 checkpoint_lvl=1, order=None):
         x_proj_weight, delta_proj_weight, out_proj_weight, out_proj_bias = _cast_proj(
             x_proj_weight, delta_proj_weight, out_proj_weight, out_proj_bias)
+        save = _saving()
         out_z, saved = _InnerCore.forward(xz, conv1d_weight, conv1d_bias, x_proj_weight, delta_proj_weight, A, B, C, D,
-                                          delta_bias, B_proj_bias, C_proj_bias, delta_softplus, order=order)
+                                          delta_bias, B_proj_bias, C_proj_bias, delta_softplus, order=order, save_states=save)
         ctx.delta_softplus = delta_softplus
         ctx.order = order
         ctx.out_proj_bias_is_None = out_proj_bias is None
-        saved = saved + (out_proj_weight, out_z)
-        _save(ctx, saved)
+        if save:
+            _save(ctx, saved + (out_proj_weight, out_z))
         return _out_proj(out_z, out_proj_weight, out_proj_bias)
 
     @staticmethod
@@ -783,7 +820,7 @@ class MambaInnerFn(torch.autograd.Function):
         return (dxz, dcw, dcb, dxw, ddw, dout_proj_w, dout_proj_b, dA, None, None, dD, ddb, None, None, None, None, None)
 
 
-class BiMambaInnerFn(torch.autograd.Function):
+class BiMambaInnerFn(_ForwardOnlyAware):
     """selective_scan_interface.py:437-603: one conv/projection feeding a forward scan (A) and a scan over the
     flipped sequence (A_b); the flip is fused into the kernels (`reverse`) instead of materialised."""
 
@@ -794,20 +831,22 @@ class BiMambaInnerFn(torch.autograd.Function):
                 delta_softplus=True, checkpoint_lvl=1):
         x_proj_weight, delta_proj_weight, out_proj_weight, out_proj_bias = _cast_proj(
             x_proj_weight, delta_proj_weight, out_proj_weight, out_proj_bias)
+        save = _saving()
         out_f, saved = _InnerCore.forward(xz, conv1d_weight, conv1d_bias, x_proj_weight, delta_proj_weight, A, B, C, D,
-                                          delta_bias, B_proj_bias, C_proj_bias, delta_softplus)
+                                          delta_bias, B_proj_bias, C_proj_bias, delta_softplus, save_states=save)
         (xz_, conv_w, conv_b, x_dbl, xw, dw, conv_st, delta, A_, _, _, D_, db_, _xs_fx, _xs_fy) = saved
         R, N = dw.shape[1], A.shape[-1]
         d, batch, L = conv_st.shape
         x3 = x_dbl.view(-1, batch, L)
         Bm, Cm = x3[R:R + N].permute(1, 0, 2).unsqueeze(1), x3[R + N:].permute(1, 0, 2).unsqueeze(1)
         z = xz_.chunk(2, dim=1)[1]
-        out_b, xs_b, _ = selective_scan_fwd(conv_st.permute(1, 0, 2), delta, A_b, Bm, Cm, D_, z, db_, delta_softplus, reverse=True)
+        out_b, xs_b, _ = selective_scan_fwd(conv_st.permute(1, 0, 2), delta, A_b, Bm, Cm, D_, z, db_, delta_softplus, reverse=True,
+                                            save_states=save)
         out_z = out_f + out_b            # out_b is already stored in un-flipped positions
         ctx.delta_softplus = delta_softplus
         ctx.out_proj_bias_is_None = out_proj_bias is None
-        saved = saved + (out_proj_weight, out_z, A_b, xs_b.x, xs_b.y)
-        _save(ctx, saved)
+        if save:
+            _save(ctx, saved + (out_proj_weight, out_z, A_b, xs_b.x, xs_b.y))
         return _out_proj(out_z, out_proj_weight, out_proj_bias)
 
     @staticmethod
@@ -930,7 +969,7 @@ def _narrow_params(io, hid_dtype, batch, L, dims, order, weights, coord):
     return p
 
 
-class MambaNarrowFn(torch.autograd.Function):
+class MambaNarrowFn(_ForwardOnlyAware):
     """The whole narrow Mamba block, requirements/mamba_simple.py:201-270 with bimamba_type "v1" (in_proj -> mamba_inner_fn ->
     out_proj, selective_scan_interface.py:292-434), on channel-major tokens: hidden (b, d_model, l) in NATURAL token order ->
     (b, d_model, l) in natural order, scanned in `order` = (kind, H, W, nslices) or None.  Three launches forward (prologue, scan,
@@ -970,7 +1009,8 @@ class MambaNarrowFn(torch.autograd.Function):
             _lib.check(L_.mmu_mamba_narrow_pre_fwd(ct.byref(p), _stream()), "mamba_narrow_pre_fwd")
             u, delta, z = pre[:, :di], pre[:, di:2 * di], pre[:, 2 * di:3 * di]
             Bm, Cm = pre[:, 3 * di:3 * di + N].unsqueeze(1), pre[:, 3 * di + N:].unsqueeze(1)
-            out_z, xs, _ = selective_scan_fwd(u, delta, A, Bm, Cm, D, z, dt_bias, True)
+            save = _saving()
+            out_z, xs, _ = selective_scan_fwd(u, delta, A, Bm, Cm, D, z, dt_bias, True, save_states=save)
             p.out_z = out_z.data_ptr()
             if coord is not None:
                 p.coords = out.data_ptr()
@@ -982,8 +1022,9 @@ class MambaNarrowFn(torch.autograd.Function):
         ctx.conv_w_shape = conv_w.shape
         ctx.coord = None if coord is None else coord[1:]
         ctx.altho_dtype = None if altho is None else altho.dtype
-        ctx.save_for_backward(hidden, pre, out_z, xs.x, xs.y, A, D, dt_bias, coord[0] if coord is not None else None,
-                              *[w for w in weights if w is not None])
+        if save:
+            ctx.save_for_backward(hidden, pre, out_z, xs.x, xs.y, A, D, dt_bias, coord[0] if coord is not None else None,
+                                  *[w for w in weights if w is not None])
         return out
 
     @staticmethod
